@@ -2,6 +2,7 @@
 """bench.py — triangle counting on Kronecker scale-24 (edge factor 16), BASELINE.json configs[1].
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scale S] [--variant V]
+                    [--dump-outputs DIR]
 
 Our arm (default).  Untimed setup: generate the edge list with the reference generator's semantics, build the
 symmetric CSR on the GPU (radix sort), keep a copy of the CSR in PINNED host memory.  Then
@@ -29,6 +30,7 @@ and the neighbour slots of vertex range r, orients that range, and the finished 
 Reference arm (--impl reference): rank 0 only, the reference's CPU path on bounded samples of the same workload.
 """
 import argparse
+import atexit
 import ctypes
 import json
 import os
@@ -43,6 +45,11 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 REF_FULL_SCALE = 20        # the reference's complete run / our like-for-like check (about a minute of CPU time)
+# Largest k of the CPU k-clique baseline when the oracle port stands in for the reference library (kind "port").  On
+# Kronecker scale-16 with 16 host threads of a B200 machine the reference took 0.50 / 3.4 / 41 s for k = 4 / 5 / 6
+# (profiles/r2r_bench_1gpu.json) and the port 5.4 / 99.6 s for k = 4 / 5; k = 6 would keep the port busy for about
+# half an hour, so it is left out (reported in skipped_k).
+KCLIQUE_PORT_MAX_K = 5
 METRIC = "tc_edges_per_sec"
 UNIT = "edges/s"
 
@@ -59,6 +66,20 @@ os.dup2(2, 1)
 
 def emit_result(obj):
     os.write(_REAL_STDOUT, (json.dumps(obj) + "\n").encode())
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: each result the timed legs returned in their last step, as <path>/<name>.npy in float64."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, np.float64))
+    log(f"[dump] {', '.join(sorted(arrays))} -> {path}")
+
+
+def count_words(c):
+    """A count as (c >> 32, c & 0xffffffff): both words are exact in float64 whatever the count (the 8-GPU k = 7 count
+    on Kronecker scale-22, ~1.4e16, is above 2**53), so dumps of two builds differ exactly when the counts do."""
+    return [c >> 32, c & 0xffffffff]
 
 
 def peaks():
@@ -92,6 +113,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits",
                                           "-lms", "100", "-i", str(self.index)], stdout=subprocess.PIPE, text=True)
+            atexit.register(self.proc.terminate)        # a run that fails before stop() leaves no sampler behind
             threading.Thread(target=self._read, daemon=True).start()
         except Exception:
             self.proc = None
@@ -250,7 +272,9 @@ def kclique_cpu_baseline(args, G, scale=16):
     g = G.Graph.from_edgelist(src, dst, True)
     g.kclique_count(3)
     rows = []
-    for k in [k for k in kclique_sizes(args, 1) if k <= 6]:
+    sizes = [k for k in kclique_sizes(args, 1) if k <= 6]
+    skipped = [k for k in sizes if kind == "port" and k > KCLIQUE_PORT_MAX_K]
+    for k in [k for k in sizes if k not in skipped]:
         sec, cnt = dag.kclique_timed(k, 2)                     # mode 2 = edge-parallel (EP_kclisting)
         best = None
         for _ in range(3):
@@ -263,11 +287,13 @@ def kclique_cpu_baseline(args, G, scale=16):
                      "gpu_cliques_per_s": cnt / best})
         log(f"[cpu_baseline] kclique k={k} scale {scale}: {kind} {sec:.2f}s on {cores} threads, GPU {best * 1e3:.2f} ms")
     g.free()
+    if skipped:
+        log(f"[cpu_baseline] kclique k={skipped} scale {scale}: not run on the {kind} (k <= {KCLIQUE_PORT_MAX_K})")
     return {"kind": kind, "cores": cores, "unit": "cliques/s", "preprocess_seconds": pre_s,
             "sample": f"Kronecker scale-{scale} edge factor 16 (same generator), the reference's pipeline: DanischHeap "
                       f"degeneracy order -> InduceDirectedGraph -> KClique::Par::EP_kclisting on all host threads; "
                       f"gpu_seconds = gmsb_kclique_count on the same graph",
-            "results": rows}
+            "results": rows, "skipped_k": skipped}
 
 
 def run_e2e(args, G, gd, off_h, nbr_h, n, slots, m, opts, expect, world, dev):
@@ -304,7 +330,7 @@ def run_e2e(args, G, gd, off_h, nbr_h, n, slots, m, opts, expect, world, dev):
     assert all(t == expect for t in e2e_totals)
     e2e_value = m * e2e_steps / (e2e_ms * 1e-3)
 
-    return e2e_value, e2e_ms, e2e_steps, e2e_orient
+    return e2e_value, e2e_ms, e2e_steps, e2e_orient, e2e_totals[-1]
 
 
 def run_ours(args):
@@ -392,6 +418,7 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     totals = gd.allreduce_counts(parts, device=dev)
     assert all(t == expect for t in totals), (totals, expect)
+    outputs = {"triangles": count_words(totals[-1])}
     st = st0
     value = m * args.steps / (ms_total * 1e-3)
 
@@ -400,7 +427,9 @@ def run_ours(args):
     # its own vertex range of the neighbour array; h2d counts all ranks)
     e2e_value, e2e_ms, e2e_steps, e2e_orient, h2d = None, float("nan"), 1, [float("nan")], 8 * (n + 1) + 4 * slots
     if not args.no_e2e:
-        e2e_value, e2e_ms, e2e_steps, e2e_orient = run_e2e(args, G, gd, off_h, nbr_h, n, slots, m, opts, expect, world, dev)
+        e2e_value, e2e_ms, e2e_steps, e2e_orient, e2e_last = run_e2e(args, G, gd, off_h, nbr_h, n, slots, m, opts, expect,
+                                                                     world, dev)
+        outputs["e2e_triangles"] = count_words(e2e_last)
 
     # ---- roofline of the dominant kernel (k_tc_bitmap2), three views of the same launch:
     #   frac            what the formulation has to pull through the memory system — 4 B per probed list element (only the
@@ -497,7 +526,10 @@ def run_ours(args):
     # ---- the other half of BASELINE.json's metric: k-clique counts/s on configs[2] (Kronecker scale-22 ef16)
     if args.kclique:
         out["kclique"] = run_kclique(args, G, gd, rank, world, dev)
+        outputs["kclique_counts"] = [[r["k"]] + count_words(r["count"]) for r in out["kclique"]["results"]]
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         emit_result(out)
     gd.barrier()
     if torch.distributed.is_initialized():
@@ -521,7 +553,13 @@ def main():
     ap.add_argument("--no-clocks", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-CSR end-to-end leg (scale-26 runs: 8.6 GB pinned per rank)")
     ap.add_argument("--no-full-reference", action="store_true", help="reference arm: skip the complete scale-20 run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the run, write what the timed legs computed in their last step to DIR/<name>.npy "
+                         "in float64, every count c as the words (c >> 32, c & 0xffffffff): triangles, e2e_triangles, "
+                         "kclique_counts as rows of (k, high word, low word); ours only")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -2,11 +2,12 @@ import json
 import os
 import sys
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+
+from oracle.reference_cases import random_graph_edges  # noqa: E402,F401  (seeded edge lists, shared with the record)
 
 
 def pytest_configure(config):
@@ -28,13 +29,17 @@ def orc():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    """The unmodified reference behind oracle/ref_shim.cpp, when its prebuilt .so is present."""
+def ref_or_none():
+    """The reference library where it is present, else None: tests that compare with it then use the stored record."""
     from oracle import binding
-    lib = binding.reference()
-    if lib is None:
-        pytest.skip("oracle/_ref/libgmsref.so not built (needs /root/reference)")
-    return lib
+    return binding.reference()
+
+
+@pytest.fixture(scope="session")
+def reference_cases():
+    """What the reference answers on the seeded cases of the CPU suite (oracle/reference_cases.py)."""
+    from oracle import reference_cases
+    return reference_cases.load()
 
 
 @pytest.fixture(scope="session")
@@ -43,15 +48,3 @@ def gms():
     import gms_b200
     gms_b200.lib()
     return gms_b200
-
-
-def random_graph_edges(seed, n, m, skew=0.0):
-    """Seeded edge list; skew>0 concentrates endpoints on low ids (hubs)."""
-    rng = np.random.default_rng(seed)
-    if skew > 0:
-        src = np.minimum((rng.random(m) ** (1 + skew) * n).astype(np.int32), n - 1)
-        dst = np.minimum((rng.random(m) ** (1 + skew) * n).astype(np.int32), n - 1)
-    else:
-        src = rng.integers(0, n, m, dtype=np.int32)
-        dst = rng.integers(0, n, m, dtype=np.int32)
-    return src, dst

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from conftest import random_graph_edges
+from oracle import reference_cases as rc
 
 
 def rounds_from_order(order, round_of):
@@ -15,12 +16,26 @@ def rounds_from_order(order, round_of):
 
 
 @pytest.mark.parametrize("seed", range(4))
-def test_oracle_adg_matches_reference_rounds(orc, ref, seed):
-    n, m = [(60, 300), (500, 6000), (3000, 40000), (200, 8000)][seed]
-    s, d = random_graph_edges(30 + seed, n, m, skew=(seed % 2) * 1.0)
-    go, gr = orc.from_el(s, d, True), ref.from_el(s, d, True)
-    for eps in (0.0, 0.5, 1.0):
+def test_oracle_adg_matches_reference_rounds(orc, ref_or_none, reference_cases, seed):
+    """The rounds against the reference's: its stored rounds always (oracle/reference_cases.py), the library itself where
+    it is present."""
+    ref = ref_or_none
+    s, d = rc.adg_case(seed)
+    go = orc.from_el(s, d, True)
+    assert rc.adg_record(orc, None, seed) == reference_cases["adg"][seed]
+    for eps in rc.ADG_EPS:
         order_o, round_of = orc.adg_order(go, eps, False)
+        # the oracle's order visits its own rounds in sequence
+        assert (np.diff(round_of[order_o]) >= 0).all()
+        rank_o, _ = orc.adg_order(go, eps, True)
+        assert (rank_o[order_o] == np.arange(go.n)).all()
+        # quality: a (2+2eps)-approximation of the degeneracy, in the orientation the clique pipeline uses
+        degen = orc.check_degeneracy_rank(go, orc.degeneracy_rank(go))
+        later = orc.core_number_of_rank(go, (go.n - 1 - rank_o).astype(np.int32))
+        assert later <= (2 + 2 * eps) * max(degen, 1) + 1
+        if ref is None:
+            continue
+        gr = ref.from_el(s, d, True)
         order_r = ref.adg_order(gr, eps, False)
         assert sorted(order_r.tolist()) == list(range(go.n))
         # same vertices leave in the same round, and rounds come in sequence
@@ -30,23 +45,21 @@ def test_oracle_adg_matches_reference_rounds(orc, ref, seed):
         # rank format is the inverse permutation
         rank_r = ref.adg_order(gr, eps, True)
         assert (rank_r[order_r] == np.arange(go.n)).all() or True      # the two reference calls may break ties differently
-        rank_o, _ = orc.adg_order(go, eps, True)
-        assert (rank_o[order_o] == np.arange(go.n)).all()
-        # quality: a (2+2eps)-approximation of the degeneracy, in the orientation the clique pipeline uses
-        degen = orc.check_degeneracy_rank(go, orc.degeneracy_rank(go))
-        later = orc.core_number_of_rank(go, (go.n - 1 - rank_o).astype(np.int32))
-        assert later <= (2 + 2 * eps) * max(degen, 1) + 1
 
 
 @pytest.mark.parametrize("seed", range(3))
-def test_oracle_adg_boundaries_and_pull_match_reference_rounds(orc, ref, seed):
+def test_oracle_adg_boundaries_and_pull_match_reference_rounds(orc, ref_or_none, reference_cases, seed):
     """minDegree boundary and the Set (pull) form of the reference (degeneracy_approx_set.h) against the oracle: the same
-    vertices leave in the same round; push and pull are the same algorithm on the counters of the remaining vertices."""
-    n, m = [(80, 500), (600, 9000), (2500, 30000)][seed]
-    s, d = random_graph_edges(70 + seed, n, m, skew=(seed % 2) * 1.0)
+    vertices leave in the same round; push and pull are the same algorithm on the counters of the remaining vertices.
+    Against the reference's stored rounds always (oracle/reference_cases.py), the library itself where it is present."""
+    ref = ref_or_none
+    assert rc.adg_ex_record(orc, None, seed) == reference_cases["adg_ex"][seed]
+    if ref is None:
+        return
+    s, d = rc.adg_ex_case(seed)
     go, gr = orc.from_el(s, d, True), ref.from_el(s, d, True)
-    for boundary in ("average", "min"):
-        for eps in (0.0, 0.5):
+    for boundary in rc.BOUNDARIES:
+        for eps in rc.ADG_EX_EPS:
             order_o, round_of = orc.adg_order_ex(go, eps, False, boundary)
             for pull in (False, True):
                 order_r = ref.adg_order_ex(gr, eps, False, boundary, pull)

@@ -1,11 +1,13 @@
 """CPU suite: the oracle (oracle/oracle.cpp) against the golden vectors generated from the unmodified reference
-(tests/golden/make_golden.py) and, where the reference library is present, against the reference directly."""
+(tests/golden/make_golden.py), against the stored record of the reference's answers on seeded random cases
+(oracle/reference_cases.py) and, where the reference library is present, against the reference directly."""
 import hashlib
 
 import numpy as np
 import pytest
 
 from conftest import random_graph_edges
+from oracle import reference_cases as rc
 from oracle.binding import METRICS
 
 
@@ -107,11 +109,14 @@ def test_degeneracy_rank_is_valid(orc):
         assert orc.check_degeneracy_rank(g, bad) in (-1, degen)
 
 
-# ---- direct comparison with the unmodified reference (only where oracle/_ref/libgmsref.so exists) -------------------
+# ---- comparison with the unmodified reference: its stored answers always, the library itself where it is present -----
 @pytest.mark.parametrize("seed", range(6))
-def test_oracle_matches_reference_random(orc, ref, seed):
-    n, m = [(50, 200), (200, 3000), (1000, 8000), (64, 2000), (500, 500), (3000, 40000)][seed]
-    s, d = random_graph_edges(seed, n, m, skew=(seed % 3) * 0.7)
+def test_oracle_matches_reference_random(orc, ref_or_none, reference_cases, seed):
+    assert rc.random_record(orc, orc, seed) == reference_cases["random"][seed]
+    ref = ref_or_none
+    if ref is None:
+        return
+    s, d, m = rc.random_case(seed)
     go, gr = orc.from_el(s, d, True), ref.from_el(s, d, True)
     for x, y in zip(go.csr(), gr.csr()):
         assert (x == y).all()
@@ -139,18 +144,17 @@ def test_oracle_matches_reference_random(orc, ref, seed):
         assert (x == y).all()
 
 
-def test_oracle_sets_match_reference_random(orc, ref):
-    rng = np.random.default_rng(7)
-    for _ in range(200):
-        na, nb = rng.integers(0, 60, 2)
-        a = np.unique(rng.integers(0, 80, na)).astype(np.int32)
-        b = np.unique(rng.integers(0, 80, nb)).astype(np.int32)
+def test_oracle_sets_match_reference_random(orc, ref_or_none, reference_cases):
+    assert rc.set_record(orc) == reference_cases["sets"]
+    ref = ref_or_none
+    if ref is None:
+        return
+    for a, b, x in rc.set_cases():
         assert orc.intersect_count(a, b) == ref.intersect_count(a, b)
         assert orc.intersect(a, b).tolist() == ref.intersect(a, b).tolist()
         assert orc.union(a, b).tolist() == ref.union(a, b).tolist()
         assert orc.union_count(a, b) == ref.union_count(a, b)
         assert orc.difference(a, b).tolist() == ref.difference(a, b).tolist()
-        x = int(rng.integers(0, 80))
         assert orc.contains(a, x) == ref.contains(a, x)
 
 
