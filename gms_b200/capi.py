@@ -12,6 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "lib", "libgmsb.so")
 
 TC_VARIANTS = {"auto": 0, "merge": 1, "gallop": 2, "bitmap": 3}
+EDGE_PASSES = {"auto": 0, "rows": 2, "slots": 3}         # gmsb_tc_options.reserved[3]
 SIM_METRICS = {"jaccard": 0, "overlap": 1, "adamic_adar": 2, "resource": 3, "comm_neigh": 4, "total_neigh": 5,
                "pref_att": 6}
 
@@ -332,12 +333,14 @@ class Graph:
         return out.value
 
     def tc_total_ex(self, variant="auto", part_index=0, part_count=1, reuse_plan=False, hub_bitmap_bits=0,
-                    gallop_ratio=0, hub_min_work=0, item_cost=0, tile_shift=0, cta_shape=0, merge_impl=0):
-        """item_cost / tile_shift / cta_shape / merge_impl are tuning knobs carried in gmsb_tc_options.reserved[0..3]
-        (merge_impl = 1: the block-compare kernel for the balanced light pairs instead of the merge path, measured slower;
-        2 / 3: force the row-walking / the element-wise form of the schedule's edge passes)."""
+                    gallop_ratio=0, hub_min_work=0, edge_passes="auto"):
+        """Triangle count with options (gmsb_tc_options); returns (count, statistics as a dict).
+
+        With part_count > 1 the count and the statistics cover share part_index of the oriented edges.  edge_passes
+        picks the form of the schedule's two passes over the edges: "rows" walks the rows, "slots" streams over the
+        edge slots, "auto" takes the element-wise form from 4 parts on.  Both forms build the same schedule."""
         opt = TcOptions(TC_VARIANTS[variant], part_index, part_count, int(reuse_plan), hub_bitmap_bits, gallop_ratio,
-                        hub_min_work, (C.c_int32 * 4)(item_cost, tile_shift, cta_shape, merge_impl))
+                        hub_min_work, (C.c_int32 * 4)(0, 0, 0, EDGE_PASSES[edge_passes]))
         out, st = C.c_uint64(0), TcStats()
         _check(lib().gmsb_tc_total_ex(self.h, C.byref(opt), C.byref(out), C.byref(st)))
         return out.value, st.as_dict()

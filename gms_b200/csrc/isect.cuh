@@ -79,33 +79,6 @@ __device__ __forceinline__ uint32_t warp_merge_count(const vid_t *__restrict__ a
     return hits;
 }
 
-// Block-compare intersection (round-2 experiment, kept for A/B runs: tc.cu k_tc_merge<true>): each lane holds one element
-// of a 32-element block of A and of B; the B block is rotated past the A block with shuffles (32 x 32 comparisons in 32
-// steps), then the block with the smaller last element moves on (both when they are equal).  An A block is compared
-// with every B block it overlaps and with no other, so an element is matched at most once.  Measured slower than the
-// merge path on this workload (see tc.cu): the rotation costs 32 steps however full the blocks are.
-// per-lane partial count; caller reduces
-__device__ __forceinline__ uint32_t warp_block_count(const vid_t *__restrict__ a, int na, const vid_t *__restrict__ b,
-                                                     int nb, int lane) {
-    uint32_t hits = 0;
-    int ia = 0, ib = 0;
-    if (na == 0 || nb == 0) return 0;
-    vid_t va = ia + lane < na ? a[ia + lane] : 0x7fffffff;
-    vid_t vb = ib + lane < nb ? b[ib + lane] : -1;
-    for (;;) {
-        bool found = false;
-#pragma unroll
-        for (int r = 0; r < 32; ++r) found |= (va == __shfl_sync(0xffffffffu, vb, (lane + r) & 31));
-        hits += found;
-        const vid_t amax = __shfl_sync(0xffffffffu, va, min(31, na - 1 - ia));
-        const vid_t bmax = __shfl_sync(0xffffffffu, vb, min(31, nb - 1 - ib));
-        const bool adv_a = amax <= bmax, adv_b = bmax <= amax;
-        if (adv_a) { ia += 32; if (ia >= na) break; va = ia + lane < na ? a[ia + lane] : 0x7fffffff; }
-        if (adv_b) { ib += 32; if (ib >= nb) break; vb = ib + lane < nb ? b[ib + lane] : -1; }
-    }
-    return hits;
-}
-
 __device__ __forceinline__ unsigned long long warp_sum(unsigned long long x) {
     for (int o = 16; o; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
     return x;

@@ -67,6 +67,31 @@ __device__ __forceinline__ int plan_owner(vid_t v, int64_t n, const OwnerDeal &o
 
 __device__ __forceinline__ uint32_t len_class(eid_t len) { return len <= kShortLen ? 0u : (len <= kMidLen ? 1u : 2u); }
 
+// One edge (u,v) of the count pass, both forms: len = suffix length after v, du = d+(u); sums as in k_plan_count's acc.
+__device__ __forceinline__ void count_edge(vid_t v, eid_t len, unsigned long long du, const int32_t *__restrict__ dplus,
+                                           unsigned long long *__restrict__ cw, unsigned long long &deg2,
+                                           unsigned long long &wedges, unsigned long long &kept, unsigned long long &ku) {
+    const int dv = dplus[v];
+    deg2 += du + (unsigned long long)dv;
+    if (len > 0 && dv > 0) {
+        atomicAdd(&cw[3 * (int64_t)v + len_class(len)], (1ull << kCntShift) | (unsigned long long)len);
+        wedges += (unsigned long long)len; kept++; ku += du;
+    }
+}
+
+__device__ __forceinline__ void flush_counts(unsigned long long *__restrict__ acc, unsigned long long deg2,
+                                             unsigned long long wedges, unsigned long long kept, unsigned long long ku) {
+    for (int o = 16; o; o >>= 1) {
+        deg2 += __shfl_xor_sync(0xffffffffu, deg2, o);
+        wedges += __shfl_xor_sync(0xffffffffu, wedges, o);
+        kept += __shfl_xor_sync(0xffffffffu, kept, o);
+        ku += __shfl_xor_sync(0xffffffffu, ku, o);
+    }
+    if ((threadIdx.x & 31) == 0 && deg2) {
+        atomicAdd(&acc[0], deg2); atomicAdd(&acc[1], wedges); atomicAdd(&acc[2], kept); atomicAdd(&acc[3], ku);
+    }
+}
+
 template <int G>
 __global__ void __launch_bounds__(256)
 k_plan_count(const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, const int32_t *__restrict__ dplus,
@@ -83,24 +108,10 @@ k_plan_count(const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, const
         for (eid_t s = b + sub; s < e; s += G) {
             const vid_t v = nbr[s];
             if (od.parts > 1 && plan_owner(v, n, od) != part_index) continue;
-            const int dv = dplus[v];
-            const eid_t len = e - s - 1;
-            deg2 += du + (unsigned long long)dv;
-            if (len > 0 && dv > 0) {
-                atomicAdd(&cw[3 * (int64_t)v + len_class(len)], (1ull << kCntShift) | (unsigned long long)len);
-                wedges += (unsigned long long)len; kept++; ku += du;
-            }
+            count_edge(v, e - s - 1, du, dplus, cw, deg2, wedges, kept, ku);
         }
     }
-    for (int o = 16; o; o >>= 1) {
-        deg2 += __shfl_xor_sync(0xffffffffu, deg2, o);
-        wedges += __shfl_xor_sync(0xffffffffu, wedges, o);
-        kept += __shfl_xor_sync(0xffffffffu, kept, o);
-        ku += __shfl_xor_sync(0xffffffffu, ku, o);
-    }
-    if ((threadIdx.x & 31) == 0 && deg2) {
-        atomicAdd(&acc[0], deg2); atomicAdd(&acc[1], wedges); atomicAdd(&acc[2], kept); atomicAdd(&acc[3], ku);
-    }
+    flush_counts(acc, deg2, wedges, kept, ku);
 }
 
 // The same pass as an element-wise stream over the edge slots, given Dag::spos (position and suffix length per slot,
@@ -142,31 +153,22 @@ k_plan_count_flat(const vid_t *__restrict__ nbr, const uint32_t *__restrict__ sp
             if (v < 0 || (od.parts > 1 && plan_owner(v, n, od) != part_index)) continue;
             const eid_t len = (eid_t)(sps[q] & 0xffffu);
             const unsigned long long du = (unsigned long long)(sps[q] >> 16) + (unsigned long long)len + 1ull;
-            const int dv = dplus[v];
-            deg2 += du + (unsigned long long)dv;
-            if (len > 0 && dv > 0) {
-                atomicAdd(&cw[3 * (int64_t)v + len_class(len)], (1ull << kCntShift) | (unsigned long long)len);
-                wedges += (unsigned long long)len; kept++; ku += du;
-            }
+            count_edge(v, len, du, dplus, cw, deg2, wedges, kept, ku);
         }
     }
-    for (int o = 16; o; o >>= 1) {
-        deg2 += __shfl_xor_sync(0xffffffffu, deg2, o);
-        wedges += __shfl_xor_sync(0xffffffffu, wedges, o);
-        kept += __shfl_xor_sync(0xffffffffu, kept, o);
-        ku += __shfl_xor_sync(0xffffffffu, ku, o);
-    }
-    if ((threadIdx.x & 31) == 0 && deg2) {
-        atomicAdd(&acc[0], deg2); atomicAdd(&acc[1], wedges); atomicAdd(&acc[2], kept); atomicAdd(&acc[3], ku);
-    }
+    flush_counts(acc, deg2, wedges, kept, ku);
 }
 
 struct PlanParams {
     int variant;
     int hub_bits;
     long long hub_min_work;
-    long long item_cost;
 };
+
+// Work target of one hub item: list elements probed plus 4 per descriptor, and never less than 16 x d+(v), the cost of
+// setting and clearing the bitmap.  Half of it bought nothing at scale 24 (profiles/r2m_tile_order_sweep.jsonl: 35.2-35.3
+// ms of counting kernels, with address tiles, against 34.35 ms for this target with positional tiles).
+constexpr long long kItemCost = 262144;
 
 // Per vertex: hub or not, and into how many CTA items its descriptor group is cut.
 __global__ void k_classify(const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, int64_t n,
@@ -197,7 +199,7 @@ __global__ void k_classify(const eid_t *__restrict__ off, const vid_t *__restric
                     hub = span <= pp.hub_bits && (pp.variant == GMSB_TC_BITMAP || work >= pp.hub_min_work);
                     if (hub) {
                         const long long setup = 16ll * (long long)dv;
-                        const long long target = pp.item_cost > setup ? pp.item_cost : setup;
+                        const long long target = kItemCost > setup ? kItemCost : setup;
                         const long long cost = work + 4ll * cnt;
                         k = (cost + target - 1) / target;
                         if (k < 1) k = 1;
@@ -263,6 +265,39 @@ __global__ void k_plan_layout(int64_t n, unsigned long long *__restrict__ cw, co
     }
 }
 
+// Appends a light edge to the merge or the gallop list: one cursor bump per coalesced group of lanes.
+__device__ __forceinline__ void append_light(unsigned long long *__restrict__ cursor, uint64_t *__restrict__ l_desc,
+                                             vid_t *__restrict__ l_v, uint64_t ds, vid_t v) {
+    namespace cg = cooperative_groups;
+    cg::coalesced_group act = cg::coalesced_threads();
+    unsigned long long base = 0;
+    if (act.thread_rank() == 0) base = atomicAdd(cursor, (unsigned long long)act.size());
+    const unsigned long long i = act.shfl(base, 0) + act.thread_rank();
+    l_desc[i] = ds; l_v[i] = v;
+}
+
+// One edge (u,v) of the scatter pass, both forms: slot s of v in N+(u), len = suffix length after v, du = d+(u).  An edge
+// into a hub takes its descriptor's slot in v's segment (du is summed for bytes_bitmap); a light edge goes to the gallop
+// list when the two lists are skewed by at least `ratio`, to the merge list otherwise.
+__device__ __forceinline__ void scatter_edge(bool hub, vid_t v, eid_t s, eid_t len, unsigned long long du,
+                                             const int32_t *__restrict__ dplus, unsigned long long *__restrict__ pos,
+                                             uint64_t *__restrict__ desc, int variant, int ratio,
+                                             uint64_t *__restrict__ m_desc, vid_t *__restrict__ m_v,
+                                             uint64_t *__restrict__ g_desc, vid_t *__restrict__ g_v,
+                                             unsigned long long *__restrict__ cursors, unsigned long long &hub_u) {
+    const uint64_t ds = ((uint64_t)(s + 1) << kLenBits) | (uint64_t)len;
+    if (hub) {
+        hub_u += du;
+        desc[atomicAdd(&pos[3 * (int64_t)v + len_class(len)], 1ull)] = ds;
+        return;
+    }
+    const long long a = (long long)len, dv = dplus[v];
+    const long long lo = a < dv ? a : dv, hi = a < dv ? dv : a;
+    const bool gallop = variant == GMSB_TC_GALLOP || (variant != GMSB_TC_MERGE && hi >= (long long)ratio * lo);
+    if (gallop) append_light(&cursors[1], g_desc, g_v, ds, v);
+    else append_light(&cursors[0], m_desc, m_v, ds, v);
+}
+
 template <int G>
 __global__ void __launch_bounds__(256)
 k_plan_scatter(const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, const int32_t *__restrict__ dplus,
@@ -271,7 +306,6 @@ k_plan_scatter(const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, con
                uint64_t *__restrict__ m_desc, vid_t *__restrict__ m_v, uint64_t *__restrict__ g_desc,
                vid_t *__restrict__ g_v, unsigned long long *__restrict__ cursors /* [0]=merge [1]=gallop */,
                unsigned long long *__restrict__ acc /* [0] = sum of d+(u) over the own hub edges */) {
-    namespace cg = cooperative_groups;
     const int sub = threadIdx.x % G;
     const int64_t grp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / G;
     const int64_t ngrp = ((int64_t)gridDim.x * blockDim.x) / G;
@@ -285,28 +319,8 @@ k_plan_scatter(const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, con
             if (od.parts > 1 && plan_owner(v, n, od) != part_index) continue;
             const uint8_t state = vstate[v];
             if (state == kDead) continue;
-            const uint64_t ds = ((uint64_t)(s + 1) << kLenBits) | (uint64_t)len;
-            if (state == kHub) {
-                hub_u += (unsigned long long)(e - b);
-                desc[atomicAdd(&pos[3 * (int64_t)v + len_class(len)], 1ull)] = ds;
-                continue;
-            }
-            const long long a = (long long)len, dv = dplus[v];
-            const long long lo = a < dv ? a : dv, hi = a < dv ? dv : a;
-            const bool gallop = variant == GMSB_TC_GALLOP || (variant != GMSB_TC_MERGE && hi >= (long long)ratio * lo);
-            if (gallop) {
-                cg::coalesced_group act = cg::coalesced_threads();
-                unsigned long long base = 0;
-                if (act.thread_rank() == 0) base = atomicAdd(&cursors[1], (unsigned long long)act.size());
-                const unsigned long long i = act.shfl(base, 0) + act.thread_rank();
-                g_desc[i] = ds; g_v[i] = v;
-            } else {
-                cg::coalesced_group act = cg::coalesced_threads();
-                unsigned long long base = 0;
-                if (act.thread_rank() == 0) base = atomicAdd(&cursors[0], (unsigned long long)act.size());
-                const unsigned long long i = act.shfl(base, 0) + act.thread_rank();
-                m_desc[i] = ds; m_v[i] = v;
-            }
+            scatter_edge(state == kHub, v, s, len, (unsigned long long)(e - b), dplus, pos, desc, variant, ratio, m_desc,
+                         m_v, g_desc, g_v, cursors, hub_u);
         }
     }
     for (int o = 16; o; o >>= 1) hub_u += __shfl_xor_sync(0xffffffffu, hub_u, o);
@@ -321,7 +335,6 @@ k_plan_scatter_flat(const vid_t *__restrict__ nbr, const uint32_t *__restrict__ 
                     uint64_t *__restrict__ m_desc, vid_t *__restrict__ m_v, uint64_t *__restrict__ g_desc,
                     vid_t *__restrict__ g_v, unsigned long long *__restrict__ cursors /* [0]=merge [1]=gallop */,
                     unsigned long long *__restrict__ acc /* [0] = sum of d+(u) over the own hub edges */) {
-    namespace cg = cooperative_groups;
     unsigned long long hub_u = 0;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t s0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; s0 < m; s0 += kFlatUnroll * stride) {
@@ -341,28 +354,9 @@ k_plan_scatter_flat(const vid_t *__restrict__ nbr, const uint32_t *__restrict__ 
             if (v < 0 || len <= 0 || (od.parts > 1 && plan_owner(v, n, od) != part_index)) continue;
             const uint8_t state = vstate[v];
             if (state == kDead) continue;
-            const uint64_t ds = ((uint64_t)(s + 1) << kLenBits) | (uint64_t)len;
-            if (state == kHub) {
-                hub_u += (unsigned long long)(sps[q] >> 16) + (unsigned long long)len + 1ull;
-                desc[atomicAdd(&pos[3 * (int64_t)v + len_class(len)], 1ull)] = ds;
-                continue;
-            }
-            const long long a = (long long)len, dv = dplus[v];
-            const long long lo = a < dv ? a : dv, hi = a < dv ? dv : a;
-            const bool gallop = variant == GMSB_TC_GALLOP || (variant != GMSB_TC_MERGE && hi >= (long long)ratio * lo);
-            if (gallop) {
-                cg::coalesced_group act = cg::coalesced_threads();
-                unsigned long long base = 0;
-                if (act.thread_rank() == 0) base = atomicAdd(&cursors[1], (unsigned long long)act.size());
-                const unsigned long long i = act.shfl(base, 0) + act.thread_rank();
-                g_desc[i] = ds; g_v[i] = v;
-            } else {
-                cg::coalesced_group act = cg::coalesced_threads();
-                unsigned long long base = 0;
-                if (act.thread_rank() == 0) base = atomicAdd(&cursors[0], (unsigned long long)act.size());
-                const unsigned long long i = act.shfl(base, 0) + act.thread_rank();
-                m_desc[i] = ds; m_v[i] = v;
-            }
+            const unsigned long long du = (unsigned long long)(sps[q] >> 16) + (unsigned long long)len + 1ull;
+            scatter_edge(state == kHub, v, s, len, du, dplus, pos, desc, variant, ratio, m_desc, m_v, g_desc, g_v, cursors,
+                         hub_u);
         }
     }
     for (int o = 16; o; o >>= 1) hub_u += __shfl_xor_sync(0xffffffffu, hub_u, o);
@@ -372,13 +366,13 @@ k_plan_scatter_flat(const vid_t *__restrict__ nbr, const uint32_t *__restrict__ 
 // Order key of an item: window class, then the L2 tile its suffixes start in (tile-major order keeps the lists that
 // concurrently running CTAs stream inside the L2), then heaviest vertex first.  Window classes: 0 = NEAR (everything
 // after v, up to n-1, fits the small window: no element can fall outside the bitmap), 1 = small window, 2 = wide.
-// Two ways to name the tile (gmsb_tc_options.reserved[1]): from the slice's position inside v's descriptor segment
-// (descriptors arrive in roughly ascending u; round 1's rule, when every device had to derive the same item order
-// without looking at descriptors whose order depends on the scatter pass's atomics), or — addr_shift > 0 — from where
-// the slice's first long suffix actually starts in the neighbour array (every device orders its own share now).
+// The tile is named by the slice's position inside v's descriptor segment (descriptors arrive in roughly ascending u),
+// on a scale of ntiles = one per kTileSlots slots of the neighbour array: slices at the same relative position of
+// different hubs advance through the array together, which the L2 rewards more than tiles read off the suffixes' start
+// addresses (DESIGN.md §3.1).
 constexpr int kNearWords = kSmallWindowBytes / 4 - 1;
-__global__ void k_item_keys(const Item *__restrict__ items, int64_t cnt, int64_t n, int64_t ntiles, int addr_shift,
-                            int vbits, int tbits, const uint64_t *__restrict__ desc,
+constexpr int64_t kTileSlots = int64_t(1) << 24;
+__global__ void k_item_keys(const Item *__restrict__ items, int64_t cnt, int64_t n, int64_t ntiles, int vbits, int tbits,
                             const int64_t *__restrict__ nitems, const int64_t *__restrict__ item_base,
                             const eid_t *__restrict__ off, const vid_t *__restrict__ nbr,
                             uint64_t *__restrict__ keys, unsigned long long *__restrict__ cls_count /* 3 */,
@@ -386,12 +380,7 @@ __global__ void k_item_keys(const Item *__restrict__ items, int64_t cnt, int64_t
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < cnt; i += (int64_t)gridDim.x * blockDim.x) {
         const Item it = items[i];
         const int64_t k = nitems[it.v], j = i - item_base[it.v];
-        uint64_t tile = (uint64_t)(j * ntiles / k);
-        if (addr_shift > 0) {
-            // the long suffixes carry the work: first descriptor of the longest class present in the slice
-            const int first = it.n1 < it.count ? it.n1 : (it.n0 < it.count ? it.n0 : 0);
-            tile = (desc[it.begin + first] >> kLenBits) >> addr_shift;
-        }
+        const uint64_t tile = (uint64_t)(j * ntiles / k);
         int words = (int)(((int64_t)nbr[off[it.v + 1] - 1] - it.v + 31) >> 5);
         // a NEAR window starts at the multiple of 32 at or below v + 1 and holds every id up to n - 1
         const int64_t reach_words = ((n - 1 - (((int64_t)it.v + 1) & ~int64_t(31))) >> 5) + 1;
@@ -413,82 +402,18 @@ __global__ void k_item_keys(const Item *__restrict__ items, int64_t cnt, int64_t
 // descriptors from shared-memory tickets, one per length class (suffix lengths vary by 1000x): a lane, an 8-lane
 // group or the whole warp takes one descriptor, so short suffixes do not pay a warp's worth of control overhead.
 // List elements are read with coalesced, 4-deep predicated loads and cost ONE branch-free probe each:
-// out-of-window elements (and predicated-off slots, x = ~0) are clamped onto the always-zero guard word.
+// out-of-window elements and predicated-off slots are pointed at the always-zero guard word.
 constexpr int kDescChunk = 4;
 
-// G lanes cooperate on one descriptor; the warp takes 32/G descriptors per ticket (4 when G == 32).
-template <int G, bool DEEP = false>
-__device__ __forceinline__ uint32_t stream_class(const uint64_t *__restrict__ dptr, int lo, int hi, int *ticket,
-                                                 const vid_t *__restrict__ nbr, const uint32_t *bm, uint32_t base,
-                                                 uint32_t cap_words, int lane) {
-    uint32_t hits = 0;
-    if (lo >= hi) return 0;
-    constexpr int BATCH = G == 32 ? kDescChunk : 32 / G;
-    for (;;) {
-        int d0 = 0;
-        if (lane == 0) d0 = atomicAdd(ticket, BATCH);
-        d0 = __shfl_sync(0xffffffffu, d0, 0) + lo;
-        if (d0 >= hi) break;
-        if constexpr (G == 32) {
-            const int nd = min(BATCH, hi - d0);
-            const uint64_t mine = lane < nd ? __ldcs(&dptr[d0 + lane]) : 0ull;
-            for (int k = 0; k < nd; ++k) {
-                const uint64_t ds = __shfl_sync(0xffffffffu, mine, k);
-                const vid_t *__restrict__ p = nbr + (ds >> kLenBits);
-                const int len = (int)(ds & kLenMask);
-                if constexpr (DEEP) {
-                    for (int j = lane; j < len; j += 256) {       // 8 loads in flight per lane
-                        uint32_t x[8];
-#pragma unroll
-                        for (int q = 0; q < 8; ++q) x[q] = j + 32 * q < len ? (uint32_t)p[j + 32 * q] - base : ~0u;
-#pragma unroll
-                        for (int q = 0; q < 8; ++q) hits += probe(bm, x[q], cap_words);
-                    }
-                } else {
-                    for (int j = lane; j < len; j += 128) {
-                        const uint32_t x0 = (uint32_t)p[j] - base;
-                        const uint32_t x1 = j + 32 < len ? (uint32_t)p[j + 32] - base : ~0u;
-                        const uint32_t x2 = j + 64 < len ? (uint32_t)p[j + 64] - base : ~0u;
-                        const uint32_t x3 = j + 96 < len ? (uint32_t)p[j + 96] - base : ~0u;
-                        hits += probe(bm, x0, cap_words) + probe(bm, x1, cap_words) + probe(bm, x2, cap_words) +
-                                probe(bm, x3, cap_words);
-                    }
-                }
-            }
-        } else {
-            const int idx = d0 + lane / G, sub = lane % G;
-            const uint64_t ds = idx < hi ? __ldcs(&dptr[idx]) : 0ull;
-            const vid_t *__restrict__ p = nbr + (ds >> kLenBits);
-            const int len = (int)(ds & kLenMask);
-            if constexpr (G == 1) {
-#pragma unroll
-                for (int j = 0; j < kShortLen; ++j)
-                    hits += probe(bm, j < len ? (uint32_t)p[j] - base : ~0u, cap_words);
-            } else {
-                for (int j = sub; j < len; j += 4 * G) {
-                    const uint32_t x0 = (uint32_t)p[j] - base;
-                    const uint32_t x1 = j + G < len ? (uint32_t)p[j + G] - base : ~0u;
-                    const uint32_t x2 = j + 2 * G < len ? (uint32_t)p[j + 2 * G] - base : ~0u;
-                    const uint32_t x3 = j + 3 * G < len ? (uint32_t)p[j + 3 * G] - base : ~0u;
-                    hits += probe(bm, x0, cap_words) + probe(bm, x1, cap_words) + probe(bm, x2, cap_words) +
-                            probe(bm, x3, cap_words);
-                }
-            }
-        }
-    }
-    return hits;
-}
-
-// ---- round-2 form of the streaming loops ---------------------------------------------------------------------------
-// Same schedule, fewer instructions per probe (the kernel is issue-bound: 72 % issue-active, 20.7 warp instructions per
-// 32 probes in round 1):
+// The streaming loops take fewer instructions per probe than round 1's (which were issue-bound: 72 % issue-active, 20.7
+// warp instructions per 32 probes; 33.7 ms against 32.0 ms at scale 24, DESIGN.md §3.1):
 //   * NEAR items — hubs whose whole possible range (v, n-1] fits the window, which is where 99 % of the work is (hubs
 //     are the last vertices in rank space) — need no clamp: every element of a suffix is inside the bitmap, and slots
 //     that are predicated off are pointed at the guard word with a constant instead of a min;
 //   * the long-suffix loop runs its full 128-element blocks without per-element bounds (one predicated tail block);
 //   * the bit is taken with a wrapping funnel shift (no `& 31`).
-// VEC adds the 128-bit form the north star asks to compare: scalar head up to the first 16-byte boundary, int4 body,
-// scalar tail.
+// 128-bit loads do not pay here: a suffix starts at an arbitrary 4-byte offset, and the scalar head and tail an int4 body
+// needs cost more issue slots than they save (37.7 ms against 32.0 ms, DESIGN.md §3.1).
 //     In a NEAR item the window starts at a multiple of 32 (base = (v + 1) & ~31), so the bit number inside a word is
 //     the element's own low five bits and the subtraction of the base moves into the (per-item) bitmap pointer:
 //     element e -> word (bm - base / 32)[e >> 5], bit e & 31.  SASS per probe: LDG, SHF, LOP3, LDS, SHF.W, LOP3 + IADD3 / 2.
@@ -502,7 +427,8 @@ __device__ __forceinline__ uint32_t probe2(const uint32_t *bm, uint32_t e, uint3
     }
 }
 
-template <int G, bool NEAR, bool VEC>
+// G lanes cooperate on one descriptor; the warp takes 32/G descriptors per ticket (4 when G == 32).
+template <int G, bool NEAR>
 __device__ __forceinline__ uint32_t stream_class2(const uint64_t *__restrict__ dptr, int lo, int hi, int *ticket,
                                                   const vid_t *__restrict__ nbr, const uint32_t *bm, uint32_t base,
                                                   uint32_t cap_words, int lane) {
@@ -521,56 +447,23 @@ __device__ __forceinline__ uint32_t stream_class2(const uint64_t *__restrict__ d
             const uint64_t mine = lane < nd ? __ldcs(&dptr[d0 + lane]) : 0ull;
             for (int k = 0; k < nd; ++k) {
                 const uint64_t ds = __shfl_sync(0xffffffffu, mine, k);
-                const int64_t start = (int64_t)(ds >> kLenBits);
-                const vid_t *__restrict__ p = nbr + start;
-                int len = (int)(ds & kLenMask);
-                if constexpr (VEC) {
-                    const int head = min(len, (int)((4 - (start & 3)) & 3));      // scalars before the 16-byte boundary
-                    if (head) {
-                        const uint32_t x = lane < head ? (uint32_t)p[lane] : off_x;
-                        hits += probe2<NEAR>(bm, x, base, cap_words);
-                    }
-                    const int4 *__restrict__ pv = reinterpret_cast<const int4 *>(p + head);
-                    const int nvec = (len - head) >> 2;
-                    int i = lane;
-                    for (; i + 32 <= (nvec & ~31) + lane; i += 32) {             // full rounds: 32 x int4 = 128 elements
-                        const int4 q = pv[i];
-                        hits += probe2<NEAR>(bm, (uint32_t)q.x, base, cap_words) +
-                                probe2<NEAR>(bm, (uint32_t)q.y, base, cap_words) +
-                                probe2<NEAR>(bm, (uint32_t)q.z, base, cap_words) +
-                                probe2<NEAR>(bm, (uint32_t)q.w, base, cap_words);
-                    }
-                    if (nvec & 31) {
-                        const bool ok = i < nvec;
-                        int4 q = make_int4(0, 0, 0, 0);
-                        if (ok) q = pv[i];
-                        hits += probe2<NEAR>(bm, ok ? (uint32_t)q.x : off_x, base, cap_words) +
-                                probe2<NEAR>(bm, ok ? (uint32_t)q.y : off_x, base, cap_words) +
-                                probe2<NEAR>(bm, ok ? (uint32_t)q.z : off_x, base, cap_words) +
-                                probe2<NEAR>(bm, ok ? (uint32_t)q.w : off_x, base, cap_words);
-                    }
-                    const int done = head + (nvec << 2);
-                    if (done < len) {
-                        const uint32_t x = done + lane < len ? (uint32_t)p[done + lane] : off_x;
-                        hits += probe2<NEAR>(bm, x, base, cap_words);
-                    }
-                } else {
-                    const vid_t *__restrict__ q = p + lane;
-                    for (int t = len >> 7; t > 0; --t, q += 128) {               // full 128-element blocks, no bounds
-                        const uint32_t x0 = (uint32_t)q[0], x1 = (uint32_t)q[32],
-                                       x2 = (uint32_t)q[64], x3 = (uint32_t)q[96];
-                        hits += probe2<NEAR>(bm, x0, base, cap_words) + probe2<NEAR>(bm, x1, base, cap_words) +
-                                probe2<NEAR>(bm, x2, base, cap_words) + probe2<NEAR>(bm, x3, base, cap_words);
-                    }
-                    const int rem = len & 127;
-                    if (rem) {
-                        const uint32_t x0 = lane < rem ? (uint32_t)q[0] : off_x;
-                        const uint32_t x1 = lane + 32 < rem ? (uint32_t)q[32] : off_x;
-                        const uint32_t x2 = lane + 64 < rem ? (uint32_t)q[64] : off_x;
-                        const uint32_t x3 = lane + 96 < rem ? (uint32_t)q[96] : off_x;
-                        hits += probe2<NEAR>(bm, x0, base, cap_words) + probe2<NEAR>(bm, x1, base, cap_words) +
-                                probe2<NEAR>(bm, x2, base, cap_words) + probe2<NEAR>(bm, x3, base, cap_words);
-                    }
+                const vid_t *__restrict__ p = nbr + (ds >> kLenBits);
+                const int len = (int)(ds & kLenMask);
+                const vid_t *__restrict__ q = p + lane;
+                for (int t = len >> 7; t > 0; --t, q += 128) {               // full 128-element blocks, no bounds
+                    const uint32_t x0 = (uint32_t)q[0], x1 = (uint32_t)q[32],
+                                   x2 = (uint32_t)q[64], x3 = (uint32_t)q[96];
+                    hits += probe2<NEAR>(bm, x0, base, cap_words) + probe2<NEAR>(bm, x1, base, cap_words) +
+                            probe2<NEAR>(bm, x2, base, cap_words) + probe2<NEAR>(bm, x3, base, cap_words);
+                }
+                const int rem = len & 127;
+                if (rem) {
+                    const uint32_t x0 = lane < rem ? (uint32_t)q[0] : off_x;
+                    const uint32_t x1 = lane + 32 < rem ? (uint32_t)q[32] : off_x;
+                    const uint32_t x2 = lane + 64 < rem ? (uint32_t)q[64] : off_x;
+                    const uint32_t x3 = lane + 96 < rem ? (uint32_t)q[96] : off_x;
+                    hits += probe2<NEAR>(bm, x0, base, cap_words) + probe2<NEAR>(bm, x1, base, cap_words) +
+                            probe2<NEAR>(bm, x2, base, cap_words) + probe2<NEAR>(bm, x3, base, cap_words);
                 }
             }
         } else {
@@ -597,8 +490,7 @@ __device__ __forceinline__ uint32_t stream_class2(const uint64_t *__restrict__ d
     return hits;
 }
 
-// VAR 0: the round-1 loops (stream_class); 1: stream_class2; 2: stream_class2 with the 128-bit body
-template <int BLOCK, int MINB, int VAR, bool NEAR>
+template <int BLOCK, int MINB, bool NEAR>
 __global__ void __launch_bounds__(BLOCK, MINB)
 k_tc_bitmap2(const Item *__restrict__ items, int64_t count, uint32_t cap_words,
              const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, const uint64_t *__restrict__ desc,
@@ -625,55 +517,10 @@ k_tc_bitmap2(const Item *__restrict__ items, int64_t count, uint32_t cap_words,
         }
         __syncthreads();                              // bitmap of N+(v) complete
         const uint64_t *__restrict__ dptr = desc + item.begin;
-        uint32_t hits;
-        if constexpr (VAR == 0) {
-            hits = stream_class<32>(dptr, item.n1, item.count, &s_next[2], nbr, bm, base, cap_words, lane);
-            hits += stream_class<8>(dptr, item.n0, item.n1, &s_next[1], nbr, bm, base, cap_words, lane);
-            hits += stream_class<1>(dptr, 0, item.n0, &s_next[0], nbr, bm, base, cap_words, lane);
-        } else {
-            const uint32_t *bmv = NEAR ? bm - (base >> 5) : bm;       // NEAR: indexed by the element's own word number
-            hits = stream_class2<32, NEAR, VAR == 2>(dptr, item.n1, item.count, &s_next[2], nbr, bmv, base, cap_words, lane);
-            hits += stream_class2<8, NEAR, false>(dptr, item.n0, item.n1, &s_next[1], nbr, bmv, base, cap_words, lane);
-            hits += stream_class2<1, NEAR, false>(dptr, 0, item.n0, &s_next[0], nbr, bmv, base, cap_words, lane);
-        }
-        hits64 += hits;
-        __syncthreads();                              // every probe of this item done
-        for (eid_t j = ob + tid; j < oe; j += BLOCK) bm[((uint32_t)nbr[j] - base) >> 5] = 0u;
-    }
-    unsigned long long s = block_sum(hits64, red);
-    if (tid == 0 && s) atomicAdd(total, s);
-}
-
-template <int BLOCK, int MINB, bool DEEP = false>
-__global__ void __launch_bounds__(BLOCK, MINB)
-k_tc_bitmap(const Item *__restrict__ items, int64_t count, uint32_t cap_words,
-            const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, const uint64_t *__restrict__ desc,
-            unsigned long long *__restrict__ total, unsigned int *__restrict__ ticket) {
-    extern __shared__ uint32_t bm[];                  // cap_words + 1 words
-    __shared__ unsigned long long red[BLOCK / 32];
-    __shared__ unsigned int s_item;
-    __shared__ int s_next[3];
-    const int tid = threadIdx.x, lane = tid & 31;
-    for (uint32_t i = tid; i <= cap_words; i += BLOCK) bm[i] = 0u;
-    unsigned long long hits64 = 0;
-    for (;;) {
-        if (tid == 0) { s_item = atomicAdd(ticket, 1u); s_next[0] = 0; s_next[1] = 0; s_next[2] = 0; }
-        __syncthreads();                              // ticket visible; previous item's clears done
-        const int64_t it = (int64_t)s_item;
-        if (it >= count) break;
-        const Item item = items[it];                                      // plan order: L2 tile, then heaviest
-        const vid_t v = item.v;
-        const eid_t ob = off[v], oe = off[v + 1];
-        const uint32_t base = (uint32_t)v + 1u;
-        for (eid_t j = ob + tid; j < oe; j += BLOCK) {
-            const uint32_t x = (uint32_t)nbr[j] - base;
-            atomicOr(&bm[x >> 5], 1u << (x & 31));
-        }
-        __syncthreads();                              // bitmap of N+(v) complete
-        const uint64_t *__restrict__ dptr = desc + item.begin;
-        uint32_t hits = stream_class<32, DEEP>(dptr, item.n1, item.count, &s_next[2], nbr, bm, base, cap_words, lane);
-        hits += stream_class<8>(dptr, item.n0, item.n1, &s_next[1], nbr, bm, base, cap_words, lane);
-        hits += stream_class<1>(dptr, 0, item.n0, &s_next[0], nbr, bm, base, cap_words, lane);
+        const uint32_t *bmv = NEAR ? bm - (base >> 5) : bm;           // NEAR: indexed by the element's own word number
+        uint32_t hits = stream_class2<32, NEAR>(dptr, item.n1, item.count, &s_next[2], nbr, bmv, base, cap_words, lane);
+        hits += stream_class2<8, NEAR>(dptr, item.n0, item.n1, &s_next[1], nbr, bmv, base, cap_words, lane);
+        hits += stream_class2<1, NEAR>(dptr, 0, item.n0, &s_next[0], nbr, bmv, base, cap_words, lane);
         hits64 += hits;
         __syncthreads();                              // every probe of this item done
         for (eid_t j = ob + tid; j < oe; j += BLOCK) bm[((uint32_t)nbr[j] - base) >> 5] = 0u;
@@ -702,19 +549,18 @@ k_tc_gallop(const uint64_t *__restrict__ desc, const vid_t *__restrict__ vs,
     if (threadIdx.x == 0 && s) atomicAdd(total, s);
 }
 
-// Balanced light pairs, one warp per edge.  BLOCK = false (default): merge path — lists staged through shared memory,
-// every lane walks a share of the merge diagonal; true (gmsb_tc_options.reserved[3] = 1, A/B runs): the block-compare
-// intersection of isect.cuh, which was measured SLOWER (scale 24, every edge forced through this kernel: 1066 ms
-// against 534 ms; light edges of the auto schedule 3.59 against 3.19 ms): its 32-step rotation costs the same for a
-// block of three elements as for a full one, and the light lists are short.
+// Balanced light pairs, one warp per edge: merge path — lists staged through shared memory, every lane walks a share of
+// the merge diagonal.  A block-compare intersection (32 x 32 comparisons by rotating one block past the other) was
+// measured slower (scale 24, every edge forced through this kernel: 1066 ms against 534 ms; light edges of the auto
+// schedule 3.59 against 3.19 ms): its 32-step rotation costs the same for a block of three elements as for a full one,
+// and the light lists are short.
 constexpr int kMergeWarps = 8;
 
-template <bool BLOCK>
 __global__ void __launch_bounds__(kMergeWarps * 32)
 k_tc_merge(const uint64_t *__restrict__ desc, const vid_t *__restrict__ vs,
            int64_t count, const eid_t *__restrict__ off, const vid_t *__restrict__ nbr,
            unsigned long long *__restrict__ total) {
-    __shared__ vid_t stage[BLOCK ? 1 : kMergeWarps][BLOCK ? 1 : kMergeTile + 2];
+    __shared__ vid_t stage[kMergeWarps][kMergeTile + 2];
     __shared__ unsigned long long red[kMergeWarps];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
@@ -724,11 +570,8 @@ k_tc_merge(const uint64_t *__restrict__ desc, const vid_t *__restrict__ vs,
         const uint64_t ds = desc[i];
         const vid_t v = vs[i];
         const eid_t ob = off[v];
-        if constexpr (BLOCK)
-            hits += warp_block_count(nbr + (ds >> kLenBits), (int)(ds & kLenMask), nbr + ob, (int)(off[v + 1] - ob), lane);
-        else
-            hits += warp_merge_count(nbr + (ds >> kLenBits), (int)(ds & kLenMask), nbr + ob, (int)(off[v + 1] - ob), lane,
-                                     stage[wib]);
+        hits += warp_merge_count(nbr + (ds >> kLenBits), (int)(ds & kLenMask), nbr + ob, (int)(off[v + 1] - ob), lane,
+                                 stage[wib]);
     }
     unsigned long long s = block_sum(hits, red);
     if (threadIdx.x == 0 && s) atomicAdd(total, s);
@@ -742,14 +585,17 @@ gmsb_tc_options normalise(const gmsb_tc_options *in) {
     if (o.hub_bitmap_bits <= 0) o.hub_bitmap_bits = 512 * 1024;      // 64 KB of shared memory
     if (o.gallop_ratio <= 0) o.gallop_ratio = 8;
     if (o.hub_min_work <= 0) o.hub_min_work = 1024;
+    GMSB_REQUIRE(o.reserved[0] == 0 && o.reserved[1] == 0 && o.reserved[2] == 0 &&
+                     (o.reserved[3] == 0 || o.reserved[3] == 2 || o.reserved[3] == 3),
+                 "tc: reserved[0..2] must be 0 and reserved[3] one of 0, 2, 3");
     return o;
 }
 
 bool same_plan(const gmsb_tc_options &a, const gmsb_tc_options &b) {
     return a.variant == b.variant && a.hub_bitmap_bits == b.hub_bitmap_bits && a.gallop_ratio == b.gallop_ratio &&
-           a.hub_min_work == b.hub_min_work && a.reserved[0] == b.reserved[0] && a.reserved[1] == b.reserved[1] &&
-           a.part_index == b.part_index && a.part_count == b.part_count;      // a schedule holds one device's share
-    // (reserved[2], reserved[3] pick kernel builds, not the schedule)
+           a.hub_min_work == b.hub_min_work && a.part_index == b.part_index &&
+           a.part_count == b.part_count;      // a schedule holds one device's share
+    // (reserved[3] picks the form of the edge passes, and both forms build the same schedule)
 }
 
 TcPlan *build_plan(Dag &d, const gmsb_tc_options &opt) {
@@ -777,7 +623,7 @@ TcPlan *build_plan(Dag &d, const gmsb_tc_options &opt) {
         DevBuf<int> mx(2);
         cw.zero(); acc.zero(); cls.zero(); mx.zero();
         // element-wise passes from 4 parts on (lists shorter than 65536), row walks otherwise;
-        // reserved[3]: 2 forces the row walks, 3 the element-wise form (A/B runs, tests)
+        // reserved[3]: 2 forces the row walks, 3 the element-wise form
         const bool flat = d.max_dplus < 65536 && opt.reserved[3] != 2 && (opt.part_count >= 4 || opt.reserved[3] == 3);
         if (flat && d.spos.p == nullptr) {              // once per DAG
             d.spos.alloc(m);
@@ -792,8 +638,7 @@ TcPlan *build_plan(Dag &d, const gmsb_tc_options &opt) {
         tr.mark("plan: count pass");
         DevBuf<int64_t> nitems(n + 1), seg(n + 1), item_base(n + 1), segbase(n + 1);
         DevBuf<uint8_t> vstate(n);
-        PlanParams pp{opt.variant, hub_bits, (long long)opt.hub_min_work,
-                      opt.reserved[0] > 0 ? (long long)opt.reserved[0] : 262144ll};
+        PlanParams pp{opt.variant, hub_bits, (long long)opt.hub_min_work};
         k_classify<<<grid_for(n + 1, 256), 256, 0, r.stream>>>(d.off.p, d.nbr.p, n, cw.p, pp, pi, od, nitems.p, seg.p,
                                                               cls.p, mx.p, vstate.p);
         launched();
@@ -848,20 +693,16 @@ TcPlan *build_plan(Dag &d, const gmsb_tc_options &opt) {
             // order: tile-major, heaviest first inside a tile
             DevBuf<uint64_t> ik(p->n_items), ik2(p->n_items);
             DevBuf<Item> items2(p->n_items);
-            // reserved[1]: 0 = default; < 0 = no tiles; 1..63 = positional tiles of 2^x slots; 64 + x = address tiles
-            const int knob = opt.reserved[1];
-            const int addr_shift = knob >= 64 ? knob - 64 : 0;
-            const int tile_shift = knob >= 64 ? 0 : (knob > 0 ? knob : (knob < 0 ? 0 : 24));
-            const int64_t ntiles = tile_shift > 0 ? std::max<int64_t>(1, (m + (int64_t(1) << tile_shift) - 1) >> tile_shift) : 1;
+            const int64_t ntiles = std::max<int64_t>(1, (m + kTileSlots - 1) / kTileSlots);
             DevBuf<unsigned long long> ccnt(3);
             DevBuf<int> cwords(3);
             ccnt.zero(); cwords.zero();
             const int vbits = bits_for((uint64_t)n);
-            const int tbits = bits_for((uint64_t)(addr_shift > 0 ? (m >> addr_shift) : ntiles - 1));
+            const int tbits = bits_for((uint64_t)(ntiles - 1));
             const int key_bits = 2 + tbits + vbits;                 // class | tile | n - 1 - v
-            k_item_keys<<<grid_for(p->n_items, 256), 256, 0, r.stream>>>(p->items.p, p->n_items, n, ntiles, addr_shift, vbits,
-                                                                        tbits, p->desc.p, nitems.p, item_base.p, d.off.p,
-                                                                        d.nbr.p, ik.p, ccnt.p, cwords.p);
+            k_item_keys<<<grid_for(p->n_items, 256), 256, 0, r.stream>>>(p->items.p, p->n_items, n, ntiles, vbits, tbits,
+                                                                        nitems.p, item_base.p, d.off.p, d.nbr.p, ik.p,
+                                                                        ccnt.p, cwords.p);
             launched();
             unsigned long long h_cc[3];
             ccnt.download(h_cc, 3);
@@ -939,40 +780,17 @@ void tc_total(Graph &g, const gmsb_tc_options &opt_in, uint64_t *out, gmsb_tc_st
                                                   p.desc.p, total.p, ticket);
             launched();
         };
-        // One persistent wave per window class.  reserved[2] (A/B runs): 0 = round-2 loops, 7 = round-2 loops with the
-        // 128-bit body, 8 = round-1 loops; 1..6 = round-1 kernel with one launch and another CTA shape.
-        const int shape = opt.reserved[2];
         const Item *it0 = p.items.p, *it1 = it0 + p.cls_items[0], *it2 = it1 + p.cls_items[1];
-        const int wsmall = std::max(p.cls_words[0], p.cls_words[1]);
-        if (shape == 0) {
-            launch(k_tc_bitmap2<512, 4, 1, true>, 512, it0, p.cls_items[0], p.cls_words[0], tickets.p);
-            launch(k_tc_bitmap2<512, 4, 1, false>, 512, it1, p.cls_items[1], p.cls_words[1], tickets.p + 1);
-            launch(k_tc_bitmap2<512, 3, 1, false>, 512, it2, p.cls_items[2], p.cls_words[2], tickets.p + 2);
-        } else if (shape == 7) {
-            launch(k_tc_bitmap2<512, 4, 2, true>, 512, it0, p.cls_items[0], p.cls_words[0], tickets.p);
-            launch(k_tc_bitmap2<512, 4, 2, false>, 512, it1, p.cls_items[1], p.cls_words[1], tickets.p + 1);
-            launch(k_tc_bitmap2<512, 3, 2, false>, 512, it2, p.cls_items[2], p.cls_words[2], tickets.p + 2);
-        } else if (shape == 8) {
-            // small windows (<= 55 KB of bitmap): four CTAs of 512 threads per SM = 64 resident warps; wide: three
-            launch(k_tc_bitmap<512, 4>, 512, it0, p.cls_items[0] + p.cls_items[1], wsmall, tickets.p);
-            launch(k_tc_bitmap<512, 3>, 512, it2, p.cls_items[2], p.cls_words[2], tickets.p + 1);
-        } else if (shape == 1) launch(k_tc_bitmap<256, 6>, 256, p.items.p, p.n_items, p.max_span_words, tickets.p);
-        else if (shape == 2) launch(k_tc_bitmap<1024, 1>, 1024, p.items.p, p.n_items, p.max_span_words, tickets.p);
-        else if (shape == 3) launch(k_tc_bitmap<512, 4>, 512, p.items.p, p.n_items, p.max_span_words, tickets.p);
-        else if (shape == 4) launch(k_tc_bitmap<256, 8>, 256, p.items.p, p.n_items, p.max_span_words, tickets.p);
-        else if (shape == 5) launch(k_tc_bitmap<512, 3, true>, 512, p.items.p, p.n_items, p.max_span_words, tickets.p);
-        else launch(k_tc_bitmap<512, 3>, 512, p.items.p, p.n_items, p.max_span_words, tickets.p);
+        // small windows (<= 55 KB of bitmap): four CTAs of 512 threads per SM = 64 resident warps; wide: three
+        launch(k_tc_bitmap2<512, 4, true>, 512, it0, p.cls_items[0], p.cls_words[0], tickets.p);
+        launch(k_tc_bitmap2<512, 4, false>, 512, it1, p.cls_items[1], p.cls_words[1], tickets.p + 1);
+        launch(k_tc_bitmap2<512, 3, false>, 512, it2, p.cls_items[2], p.cls_words[2], tickets.p + 2);
     }
     t_bm.stop();
     t_mg.start();
     if (my_merge) {
         int grid = (int)std::min<int64_t>(ceil_div(my_merge, kMergeWarps), (int64_t)r.sm_count * 16);
-        if (opt.reserved[3] == 1)
-            k_tc_merge<true><<<grid, kMergeWarps * 32, 0, r.stream>>>(p.m_desc.p, p.m_v.p, my_merge, d.off.p,
-                                                                      d.nbr.p, total.p);
-        else
-            k_tc_merge<false><<<grid, kMergeWarps * 32, 0, r.stream>>>(p.m_desc.p, p.m_v.p, my_merge, d.off.p,
-                                                                       d.nbr.p, total.p);
+        k_tc_merge<<<grid, kMergeWarps * 32, 0, r.stream>>>(p.m_desc.p, p.m_v.p, my_merge, d.off.p, d.nbr.p, total.p);
         launched();
     }
     t_mg.stop();

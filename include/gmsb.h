@@ -178,7 +178,10 @@ typedef struct {
     int32_t hub_bitmap_bits; /* bitmap kernel's shared-memory window in bits; 0 = default                     */
     int32_t gallop_ratio;    /* galloping when longer/shorter >= ratio; 0 = default                           */
     int64_t hub_min_work;    /* a vertex is a hub when its incoming wedge work >= this; 0 = default            */
-    int32_t reserved[4];
+    int32_t reserved[4];     /* [0..2] must be 0.  [3] = form of the schedule's two passes over the edges:
+                                0 = chosen from part_count (element-wise from 4 parts on), 2 = walk the rows,
+                                3 = element-wise over the edge slots.  Both forms build the same schedule.
+                                Other values fail with GMSB_ERR_INVALID.                                      */
 } gmsb_tc_options;
 
 typedef struct {

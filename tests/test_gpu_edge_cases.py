@@ -154,6 +154,20 @@ def test_degenerate_clique_sizes_and_errors(gms):
         g.pair_similarity("jaccard", [0], [99])
 
 
+def test_tc_options_reject_unknown_reserved_values(gms):
+    """gmsb_tc_options.reserved: [0..2] must be 0 and [3] one of 0, 2, 3; anything else fails instead of running some
+    other kernel or the default."""
+    import ctypes
+    s, d = clique_edges(6)
+    g = gms.Graph.from_edgelist(s, d, True)
+    lib = gms.capi.lib()
+    for reserved in ((0, 0, 7, 0), (0, 0, 0, 1)):
+        opt = gms.capi.TcOptions(0, 0, 1, 0, 0, 0, 0, (ctypes.c_int32 * 4)(*reserved))
+        out, st = ctypes.c_uint64(0), gms.capi.TcStats()
+        assert lib.gmsb_tc_total_ex(g.h, ctypes.byref(opt), ctypes.byref(out), ctypes.byref(st)) == -1, reserved   # GMSB_ERR_INVALID
+    assert g.tc_total_ex()[0] == comb(6, 3)
+
+
 def test_large_host_csr_sorted_unsorted_and_malformed(gms):
     """A host CSR of 31 M slots through gmsb_graph_from_csr: sorted lists, a few reversed lists (the one streaming check
     finds them and only then a sort is paid for), and a malformed id at the very end."""

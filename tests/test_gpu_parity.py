@@ -140,10 +140,10 @@ def test_partition_sums_to_total(kron12, golden):
             assert edges == [full[key] for key in ("edges_bitmap", "edges_merge", "edges_gallop", "bitmap_items")]
 
 
-def test_schedule_passes_element_wise_and_row_walk_agree(gms):
+def test_schedule_edge_passes_rows_and_slots_agree(gms):
     """The two edge passes of the schedule exist in two forms: walking the rows, and element-wise over the slots (the
-    default from 4 parts on; reserved[3] = 2 / 3 force one or the other).  Same counts and the same statistics, for the
-    whole schedule and for shares of it."""
+    default from 4 parts on; edge_passes = "rows" / "slots" forces one or the other).  Same counts and the same
+    statistics, for the whole schedule and for shares of it."""
     s, d = gms.generate_rmat(16)
     g = gms.Graph.from_edgelist(s, d, True)
     keys = ("triangles", "algorithmic_bytes", "wedges_checked", "edges_bitmap", "edges_merge", "edges_gallop",
@@ -151,12 +151,13 @@ def test_schedule_passes_element_wise_and_row_walk_agree(gms):
     for variant in ("auto", "bitmap", "merge"):
         for parts in (1, 3, 5):
             for p in range(parts):
-                a = g.tc_total_ex(variant=variant, part_index=p, part_count=parts, reuse_plan=2, merge_impl=3)
-                b = g.tc_total_ex(variant=variant, part_index=p, part_count=parts, reuse_plan=2, merge_impl=2)
+                a = g.tc_total_ex(variant=variant, part_index=p, part_count=parts, reuse_plan=2, edge_passes="slots")
+                b = g.tc_total_ex(variant=variant, part_index=p, part_count=parts, reuse_plan=2, edge_passes="rows")
                 c = g.tc_total_ex(variant=variant, part_index=p, part_count=parts, reuse_plan=2)
                 assert a[0] == b[0] == c[0], (variant, parts, p)
                 assert [a[1][k] for k in keys] == [b[1][k] for k in keys] == [c[1][k] for k in keys], (variant, parts, p)
-    assert g.tc_total_ex(reuse_plan=2, merge_impl=2)[0] == g.tc_total_ex(reuse_plan=2, merge_impl=3)[0] == 15656287   # SURVEY.md 8c
+    assert (g.tc_total_ex(reuse_plan=2, edge_passes="rows")[0] == g.tc_total_ex(reuse_plan=2, edge_passes="slots")[0]
+            == 15656287)   # SURVEY.md 8c
 
 
 def test_algorithmic_bytes_match_definition(kron12, orc):

@@ -33,7 +33,8 @@ def main():
         for p in range(P):
             best = None
             for _ in range(args.reps):
-                c, st = g.tc_total_ex(part_index=p, part_count=P, reuse_plan=2, merge_impl=2 if args.row_walk else 0)
+                c, st = g.tc_total_ex(part_index=p, part_count=P, reuse_plan=2,
+                                      edge_passes="rows" if args.row_walk else "auto")
                 if best is None or st["ms_orient"] + st["ms_count"] < best["ms_orient"] + best["ms_count"]:
                     best = st
             tri += c

@@ -2,8 +2,6 @@ set -x
 mkdir -p gpurun_out
 timeout 900 python -m pytest tests -m gpu -x -q > gpurun_out/r2c_pytest.log 2>&1; echo "pytest rc=$?" >> gpurun_out/r2c_pytest.log
 tail -5 gpurun_out/r2c_pytest.log
-timeout 300 python tools/tc_sweep.py --scale 24 --reps 4 --configs '[{"variant":"auto"},{"variant":"auto","cta_shape":7},{"variant":"auto","cta_shape":8}]' > gpurun_out/r2c_tc_variants.jsonl 2> gpurun_out/r2c_tc_variants.err
-cat gpurun_out/r2c_tc_variants.jsonl | cut -c1-400
 export GMSB_KCLIQUE_TRACE=1
 timeout 300 python tools/kc_prof.py 22 6 > gpurun_out/r2c_kc_s22_k6.log 2>&1
 timeout 400 python tools/kc_prof.py 20 7 > gpurun_out/r2c_kc_s20_k7.log 2>&1
