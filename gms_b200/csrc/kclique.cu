@@ -29,7 +29,6 @@
 #include "ops.cuh"
 #include "kclique_lane.cuh"
 #include <cstdlib>
-#include <cstring>
 #include <algorithm>
 #include <vector>
 
@@ -369,12 +368,7 @@ k_kclique_big(const vid_t *__restrict__ verts, const int64_t *__restrict__ item_
         if (item >= count) break;
         // item -> (vertex t, part of its second-level members): heavy vertices are cut into several items so that
         // one dense neighbourhood does not serialise on a single CTA (item_base = exclusive scan of parts)
-        int64_t lo_t = 0, hi_t = nverts;
-        while (hi_t - lo_t > 1) {
-            const int64_t mid = (lo_t + hi_t) >> 1;
-            if (item_base[mid] <= item) lo_t = mid; else hi_t = mid;
-        }
-        const int64_t t = lo_t;
+        const int64_t t = lane::item_vertex(item_base, nverts, item);
         const int part = (int)(item - item_base[t]), nparts = (int)(item_base[t + 1] - item_base[t]);
         const vid_t u = verts[t];
         const eid_t ob = off[u];
@@ -446,10 +440,10 @@ __global__ void k_degree_key(const vid_t *__restrict__ verts, int64_t cnt, const
         keys[i] = ((uint64_t)(off[u + 1] - off[u]) << 32) | (uint32_t)u;
     }
 }
-// parts[t] = number of work items vertex t is cut into; also counts the vertices above the mid-size class
+// parts[t] = number of work items vertex t is cut into (parts[cnt] = 0 ends the list for the exclusive scan)
 constexpr int kMidD = 512;
 __global__ void k_parts(const vid_t *__restrict__ verts, int64_t cnt, const eid_t *__restrict__ off,
-                        int k, int part_rows, int64_t *__restrict__ parts, int *__restrict__ nhuge) {
+                        int k, int part_rows, int64_t *__restrict__ parts) {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i <= cnt; i += (int64_t)gridDim.x * blockDim.x) {
         if (i == cnt) { parts[i] = 0; continue; }
         const vid_t u = verts[i];
@@ -458,7 +452,6 @@ __global__ void k_parts(const vid_t *__restrict__ verts, int64_t cnt, const eid_
         // (every part rebuilds the vertex's matrix, so parts are kept few: the split is only there to spread the
         // handful of densest neighbourhoods over several SMs)
         parts[i] = k <= 4 ? 1 : (d > kMidD ? (d + part_rows - 1) / part_rows : 1);
-        if (d > kMidD) atomicAdd(nhuge, 1);
     }
 }
 __global__ void k_key_vertex(const uint64_t *__restrict__ keys, int64_t cnt, vid_t *__restrict__ verts) {
@@ -466,7 +459,7 @@ __global__ void k_key_vertex(const uint64_t *__restrict__ keys, int64_t cnt, vid
         verts[i] = (vid_t)(uint32_t)keys[i];
 }
 
-// number of vertices (of the descending-degree list) above each class boundary of the lane kernels
+// number of vertices (of the descending-degree list) above each class boundary: d+ > 512, 256, 128, 64
 __global__ void k_class_counts(const vid_t *__restrict__ verts, int64_t cnt, const eid_t *__restrict__ off,
                                int *__restrict__ counts) {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < cnt; i += (int64_t)gridDim.x * blockDim.x) {
@@ -487,17 +480,272 @@ __global__ void k_list_degrees(const vid_t *__restrict__ verts, int64_t cnt, con
     }
 }
 
-// Which kernels run the d+ > 32 sub-problems: the lane-parallel ones (kclique_lane.cuh) or the warp-cooperative ones
-// above.  GMSB_KCLIQUE_IMPL=warp|lane forces one family (A/B measurements, tests); the default takes the lane
-// kernels where they are faster (measured on B200, see DESIGN.md) and supported (4 <= k <= 10).
-constexpr int kLaneMinK = 5;
-constexpr int kPairMinDefault = 128;       // k = 7, scale 20: 85.7 s (512) -> 67.5 s (256) -> 64.5 s (128)
-bool use_lane_kernels(int k) {
-    const char *e = std::getenv("GMSB_KCLIQUE_IMPL");
-    if (e && !std::strcmp(e, "warp")) return false;
-    if (k < 4 || k - 1 > lane::kMaxNeed) return false;
-    if (e && !std::strcmp(e, "lane")) return true;
-    return k >= kLaneMinK;
+// The d+ > 32 vertices in descending out-degree order, and what every class launch needs.
+struct BigVerts {
+    const vid_t *verts;
+    int64_t count;
+    int64_t bound[4];              // how many of them have d+ > 512, 256, 128, 64
+    int maxD;
+    const eid_t *off;
+    const vid_t *nbr;
+    int k, pi, P;
+    DevBuf<unsigned long long> &total;
+};
+
+// k = 3, 4, 11..16: the warp-cooperative kernel in two launches, so that the many mid-size neighbourhoods get a small
+// matrix and several CTAs per SM.  Work items: (vertex, interleaved part of its second-level members).
+void count_warp(const BigVerts &b) {
+    Runtime &r = rt();
+    DevBuf<int64_t> parts(b.count + 1), item_base(b.count + 1);
+    k_parts<<<grid_for(b.count, 256), 256, 0, r.stream>>>(b.verts, b.count, b.off, b.k, 256, parts.p); launched();
+    auto run_class = [&](int64_t first, int64_t cnt, int classD, bool huge) {
+        if (cnt == 0) return;
+        exclusive_sum(parts.p + first, item_base.p, cnt + 1);
+        const int64_t n_items = item_base.get(cnt);
+        const int W = row_words(classD);
+        const size_t need = matrix_words(classD) * 4;
+        const bool in_smem = need + 28 * 1024 <= r.smem_optin;    // static scratch (WarpScratch etc.) is <= 25 KB
+        const size_t smem = in_smem ? need : 0;
+        DevBuf<unsigned int> ticket(1);
+        ticket.zero();
+        DevBuf<uint32_t> spill;
+        auto launch = [&](auto kern, int block) {
+            if (smem > 48 * 1024)
+                GMSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            int resident = 0;
+            GMSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, block, smem));
+            GMSB_REQUIRE(resident >= 1, "kclique_count: kernel does not fit on an SM");
+            if (!in_smem) resident = 1;
+            const int grid = (int)std::min<int64_t>(n_items, (int64_t)r.sm_count * resident);
+            if (!in_smem) spill.alloc((size_t)grid * (need / 4));
+            kern<<<grid, block, smem, r.stream>>>(b.verts + first, item_base.p, cnt, n_items, b.off, b.nbr, b.k, classD,
+                                                  b.total.p, ticket.p, in_smem ? nullptr : spill.p, b.pi, b.P);
+            launched();
+            GMSB_CUDA(cudaStreamSynchronize(r.stream));
+        };
+        // the search is a chain of dependent shared-memory steps, so resident warps are what hides its latency:
+        // a big matrix fills the SM's shared memory -> one CTA of 1024 threads; mid-size ones -> 2 x 512
+        if (huge) {
+            if (W <= 32) launch(k_kclique_big<1, 1024, 1>, 1024);
+            else if (W <= 64) launch(k_kclique_big<2, 1024, 1>, 1024);
+            else launch(k_kclique_big<4, 1024, 1>, 1024);
+        } else {
+            launch(k_kclique_big<1, 512, 2>, 512);        // kMidD = 512 -> W = 16
+        }
+    };
+    run_class(0, b.bound[0], b.maxD, true);
+    run_class(b.bound[0], b.count - b.bound[0], kMidD, false);
+}
+
+// Launches of the lane kernels' classes.  The class kernels are independent (own ticket, atomics on one total), so
+// each k_kclique_lane_mid class goes to its own stream: its CTAs fill the SMs that the previous class's last items
+// leave idle, and with the sub-problems split over several GPUs those tails are a visible share of a launch.
+// GMSB_KCLIQUE_TRACE=1 (profiling aid) serialises the launches and prints the device time and clique count of every
+// class on stderr.
+class LaneClasses {
+  public:
+    explicit LaneClasses(const BigVerts &b) : b_(b), r_(rt()), trace_(std::getenv("GMSB_KCLIQUE_TRACE") != nullptr) {
+        tickets_.zero();
+        mark(nullptr, 0);
+        if (!trace_) {
+            GMSB_CUDA(cudaEventCreateWithFlags(&own_.ready, cudaEventDisableTiming));
+            GMSB_CUDA(cudaEventRecord(own_.ready, r_.stream));
+            for (auto &st : own_.aux) {
+                GMSB_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+                GMSB_CUDA(cudaStreamWaitEvent(st, own_.ready, 0));
+            }
+        }
+    }
+
+    // ticket of the d+ > 512 (k = 5, 6) or pair (k >= 7) kernel
+    unsigned int *first_ticket() { return tickets_.p; }
+
+    // end of class `name` (`vertices` vertices), launched on the library stream
+    void mark(const char *name, int64_t vertices) {
+        if (!trace_) return;
+        Mark m{nullptr, 0, name, vertices};
+        cudaEventCreate(&m.ev);
+        own_.events.push_back(m.ev);
+        cudaEventRecord(m.ev, r_.stream);
+        m.seen = b_.total.get(0);          // synchronises: per-class counts for the trace
+        marks_.push_back(m);
+    }
+
+    // vertices [first, end) of the list through k_kclique_lane_mid<NWB, BLOCK, MINB>; with rows of 3 or more words
+    // every warp gets a box for its third-level matrices
+    template <int NWB, int BLOCK, int MINB>
+    void mid(int64_t first, int64_t end, const char *name) {
+        const int cls = next_++;
+        if (end > first) {
+            auto kern = lane::k_kclique_lane_mid<NWB, BLOCK, MINB>;
+            const size_t dyn = NWB >= 3 ? (size_t)(BLOCK / 32) * sizeof(lane::WarpBox) : 0;
+            GMSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+            int resident = 0;
+            GMSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, BLOCK, dyn));
+            GMSB_REQUIRE(resident >= 1, "kclique_count: kernel does not fit on an SM");
+            const int grid = (int)std::min<int64_t>(end - first, (int64_t)r_.sm_count * resident);
+            cudaStream_t st = trace_ ? r_.stream : own_.aux[cls];
+            kern<<<grid, BLOCK, dyn, st>>>(b_.verts + first, end - first, b_.off, b_.nbr, b_.k, b_.total.p,
+                                           tickets_.p + 1 + cls, b_.pi, b_.P);
+            launched();
+        }
+        mark(name, std::max<int64_t>(end - first, 0));
+    }
+
+    // the library stream continues after every class
+    void join() {
+        if (!trace_) {
+            for (auto &st : own_.aux) {
+                GMSB_CUDA(cudaEventRecord(own_.ready, st));
+                GMSB_CUDA(cudaStreamWaitEvent(r_.stream, own_.ready, 0));
+            }
+        }
+        GMSB_CUDA(cudaStreamSynchronize(r_.stream));
+        for (size_t i = 1; i < marks_.size(); ++i) {
+            float ms = 0;
+            cudaEventElapsedTime(&ms, marks_[i - 1].ev, marks_[i].ev);
+            std::fprintf(stderr, "[gmsb kclique k=%d] %-13s vertices=%lld ms=%.3f cliques=%llu\n", b_.k, marks_[i].name,
+                         (long long)marks_[i].vertices, ms, marks_[i].seen - marks_[i - 1].seen);
+        }
+    }
+
+  private:
+    struct Mark {
+        cudaEvent_t ev;
+        unsigned long long seen;
+        const char *name;
+        int64_t vertices;
+    };
+    const BigVerts &b_;
+    Runtime &r_;
+    const bool trace_;
+    DevBuf<unsigned int> tickets_{5};          // [0] first_ticket(), [1..4] the mid classes in launch order
+    struct Owned {                             // released also when the constructor throws half-way
+        cudaStream_t aux[4] = {nullptr, nullptr, nullptr, nullptr};
+        cudaEvent_t ready = nullptr;
+        std::vector<cudaEvent_t> events;
+        ~Owned() {
+            for (auto st : aux) if (st) cudaStreamDestroy(st);
+            if (ready) cudaEventDestroy(ready);
+            for (auto ev : events) cudaEventDestroy(ev);
+        }
+    } own_;
+    int next_ = 0;
+    std::vector<Mark> marks_;
+};
+
+// k = 5, 6: d+ > 512 through k_kclique_lane_huge, one CTA per SM on vertex parts of 64 rows (CTA-wide top of the tree,
+// compact matrices below); the four classes <= 512 / 256 / 128 / 64 through k_kclique_lane_mid.
+void count_lane_huge(const BigVerts &b) {
+    Runtime &r = rt();
+    const int64_t n_huge = b.bound[0];
+    DevBuf<int64_t> parts, item_base;
+    DevBuf<lane::u64> spill;
+    LaneClasses classes(b);
+    if (n_huge) {
+        parts.alloc(n_huge + 1);
+        item_base.alloc(n_huge + 1);
+        k_parts<<<grid_for(n_huge, 256), 256, 0, r.stream>>>(b.verts, n_huge, b.off, b.k, 64, parts.p); launched();
+        exclusive_sum(parts.p, item_base.p, n_huge + 1);
+        const int64_t n_items = item_base.get(n_huge);
+        // 512 threads cap the kernel at 128 registers and it spills; 384 threads (168 registers, no spills) were 6 %
+        // faster at scale 22, k = 6
+        constexpr int BLOCK = 384;
+        auto kern = lane::k_kclique_lane_huge<BLOCK>;
+        const size_t full = lane::huge_smem_words(b.maxD, true) * 8;
+        const bool in_smem = full + 2048 <= r.smem_optin;
+        const size_t smem = in_smem ? full : lane::huge_smem_words(b.maxD, false) * 8;
+        GMSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        const int grid = (int)std::min<int64_t>(n_items, (int64_t)r.sm_count);
+        if (!in_smem) spill.alloc((size_t)grid * (size_t)b.maxD * (size_t)lane::huge_pitch(b.maxD));
+        kern<<<grid, BLOCK, smem, r.stream>>>(b.verts, item_base.p, n_huge, n_items, b.off, b.nbr, b.k, b.maxD,
+                                              b.total.p, classes.first_ticket(), in_smem ? nullptr : spill.p, b.pi, b.P);
+        launched();
+    }
+    classes.mark("huge(d+>512)", n_huge);
+    classes.mid<8, 384, 2>(b.bound[0], b.bound[1], "mid8(<=512)");
+    classes.mid<4, 256, 4>(b.bound[1], b.bound[2], "mid4(<=256)");
+    classes.mid<2, 128, 8>(b.bound[2], b.bound[3], "mid2(<=128)");
+    classes.mid<1, 128, 8>(b.bound[3], b.count, "mid1(<=64)");
+    classes.join();
+}
+
+// k = 7..10: d+ > 128 decoupled — M1 of every such vertex to global memory (k_kclique_m1_build), then (vertex, member)
+// work items through k_kclique_lane_pair, which searches through third-level matrices; those pay when five or more
+// vertices are left below u and S[i].  The classes <= 128 / 64 go through k_kclique_lane_mid.  Smallest class of the
+// pair kernel, k = 7 at scale 20: d+ > 512 85.7 s, > 256 67.5 s, > 128 64.5 s.
+void count_lane_pair(const BigVerts &b) {
+    Runtime &r = rt();
+    const int64_t n_pair = b.bound[2];
+    LaneClasses classes(b);
+    if (n_pair) {
+        // Sizes come from the (few thousand) out-degrees on the host; the vertices are processed in batches whose
+        // matrices fit kM1Budget bytes.
+        std::vector<vid_t> hv((size_t)n_pair);
+        GMSB_CUDA(cudaMemcpyAsync(hv.data(), b.verts, sizeof(vid_t) * n_pair, cudaMemcpyDeviceToHost, r.stream));
+        GMSB_CUDA(cudaStreamSynchronize(r.stream));
+        std::vector<int> hd((size_t)n_pair);
+        {
+            // out-degrees of the listed vertices (descending): two offsets each
+            DevBuf<int> dd((size_t)n_pair);
+            k_list_degrees<<<grid_for(n_pair, 256), 256, 0, r.stream>>>(b.verts, n_pair, b.off, dd.p); launched();
+            dd.download(hd.data(), (size_t)n_pair);
+        }
+        constexpr size_t kM1Budget = size_t(12) << 30;
+        constexpr int PBLOCK = 256;
+        const size_t smem2 = lane::pair_smem_words(b.maxD, PBLOCK / 32) * 8;
+        GMSB_REQUIRE(smem2 + 4096 <= r.smem_optin, "kclique_count: out-degree too large for the pair kernel");
+        auto kern2 = lane::k_kclique_lane_pair<PBLOCK>;
+        GMSB_CUDA(cudaFuncSetAttribute(kern2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
+        int resident2 = 0;
+        GMSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident2, kern2, PBLOCK, smem2));
+        GMSB_REQUIRE(resident2 >= 1, "kclique_count: pair kernel does not fit on an SM");
+        constexpr int BBLOCK = 256;
+        const size_t smem1 = ((size_t)(BBLOCK / 32) * lane::huge_pitch(b.maxD) + (size_t)((b.maxD + 1) >> 1)) * 8;
+        auto kern1 = lane::k_kclique_m1_build<BBLOCK>;
+        GMSB_CUDA(cudaFuncSetAttribute(kern1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+        DevBuf<int64_t> pair_base, m1_off;
+        DevBuf<lane::u64> m1;
+        unsigned int *ticket = classes.first_ticket();
+        int64_t t0 = 0;
+        int64_t item0 = 0;                       // global numbering of the items, for the multi-GPU deal
+        while (t0 < n_pair) {
+            std::vector<int64_t> h_m1((size_t)0), h_items((size_t)0);
+            size_t words = 0;
+            int64_t items = 0, t1 = t0;
+            while (t1 < n_pair) {
+                const size_t w = (size_t)hd[t1] * (size_t)lane::huge_pitch(hd[t1]);
+                if (t1 > t0 && (words + w) * 8 > kM1Budget) break;
+                h_m1.push_back((int64_t)words); h_items.push_back(items);
+                words += w; items += hd[t1]; ++t1;
+            }
+            h_items.push_back(items);
+            const int64_t nv = t1 - t0;
+            m1.alloc(words);
+            m1_off.alloc((size_t)nv); pair_base.alloc((size_t)nv + 1);
+            m1_off.upload(h_m1.data(), (size_t)nv);
+            pair_base.upload(h_items.data(), (size_t)nv + 1);
+            const int grid1 = (int)std::min<int64_t>(nv, (int64_t)r.sm_count * 4);
+            kern1<<<grid1, BBLOCK, smem1, r.stream>>>(b.verts, t0, nv, b.off, b.nbr, m1_off.p, m1.p, b.maxD); launched();
+            // this process's items of the batch: global item numbers congruent to pi modulo P
+            const int shift = (int)(((int64_t)b.pi - item0 % b.P + b.P) % b.P);
+            const int64_t mine = items > shift ? (items - shift + b.P - 1) / b.P : 0;
+            if (mine) {
+                GMSB_CUDA(cudaMemsetAsync(ticket, 0, sizeof(unsigned int), r.stream));
+                const int grid2 = (int)std::min<int64_t>(mine, (int64_t)r.sm_count * resident2);
+                kern2<<<grid2, PBLOCK, smem2, r.stream>>>(b.verts, t0, pair_base.p, nv, items, b.off, m1_off.p, m1.p,
+                                                          b.k, b.maxD, b.total.p, ticket, shift, b.P);
+                launched();
+            }
+            GMSB_CUDA(cudaStreamSynchronize(r.stream));      // host vectors / batch buffers are reused
+            item0 += items;
+            t0 = t1;
+        }
+    }
+    classes.mark("pair(d+>128)", n_pair);
+    classes.mid<2, 128, 8>(b.bound[2], b.bound[3], "mid2(<=128)");
+    classes.mid<1, 128, 8>(b.bound[3], b.count, "mid1(<=64)");
+    classes.join();
 }
 
 uint64_t count_on_dag(int64_t n, int64_t m, const eid_t *off, const vid_t *nbr, int k, int pi, int P) {
@@ -533,239 +781,17 @@ uint64_t count_on_dag(int64_t n, int64_t m, const eid_t *off, const vid_t *nbr, 
         if (row_words(maxD) > 128)
             throw Error(GMSB_ERR_UNSUPPORTED, "kclique_count: max out-degree " + std::to_string(maxD) +
                                                   " exceeds 4096; orient by degree or degeneracy first");
-        const bool lane_path = use_lane_kernels(k);
-        // work items: (vertex, interleaved part of its second-level members)
-        DevBuf<int64_t> parts(nb + 1), item_base(nb + 1);
-        DevBuf<int> nhuge(1);
-        nhuge.zero();
-        k_parts<<<grid_for(nb, 256), 256, 0, r.stream>>>(vb.p, nb, off, k, lane_path ? 64 : 256, parts.p, nhuge.p); launched();
-        const int64_t n_huge = nhuge.get(0);           // vertices with d+ > kMidD come first (sorted descending)
-        // two launches so that the many mid-size neighbourhoods get a small matrix and several CTAs per SM
-        auto run_class = [&](int64_t first, int64_t cnt, int classD, bool huge) {
-            if (cnt == 0) return;
-            exclusive_sum(parts.p + first, item_base.p, cnt + 1);
-            const int64_t n_items = item_base.get(cnt);
-            const int W = row_words(classD);
-            const size_t need = matrix_words(classD) * 4;
-            const bool in_smem = need + 28 * 1024 <= r.smem_optin;    // static scratch (WarpScratch etc.) is <= 25 KB
-            const size_t smem = in_smem ? need : 0;
-            DevBuf<unsigned int> ticket(1);
-            ticket.zero();
-            DevBuf<uint32_t> spill;
-            auto launch = [&](auto kern, int block) {
-                if (smem > 48 * 1024)
-                    GMSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                int resident = 0;
-                GMSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, block, smem));
-                GMSB_REQUIRE(resident >= 1, "kclique_count: kernel does not fit on an SM");
-                if (!in_smem) resident = 1;
-                const int grid = (int)std::min<int64_t>(n_items, (int64_t)r.sm_count * resident);
-                if (!in_smem) spill.alloc((size_t)grid * (need / 4));
-                kern<<<grid, block, smem, r.stream>>>(vb.p + first, item_base.p, cnt, n_items, off, nbr, k, classD,
-                                                          total.p, ticket.p, in_smem ? nullptr : spill.p, pi, P);
-                launched();
-                GMSB_CUDA(cudaStreamSynchronize(r.stream));
-            };
-            // the search is a chain of dependent shared-memory steps, so resident warps are what hides its latency:
-            // a big matrix fills the SM's shared memory -> one CTA of 1024 threads; mid-size ones -> 2 x 512
-            if (huge) {
-                if (W <= 32) launch(k_kclique_big<1, 1024, 1>, 1024);
-                else if (W <= 64) launch(k_kclique_big<2, 1024, 1>, 1024);
-                else launch(k_kclique_big<4, 1024, 1>, 1024);
-            } else {
-                launch(k_kclique_big<1, 512, 2>, 512);        // kMidD = 512 -> W = 16
-            }
-        };
-        if (lane_path) {
-            DevBuf<int> cc(4);
-            cc.zero();
-            k_class_counts<<<grid_for(nb, 256), 256, 0, r.stream>>>(vb.p, nb, off, cc.p); launched();
-            int bound[4];
-            cc.download(bound, 4);
-            DevBuf<unsigned int> tickets(5);
-            tickets.zero();
-            // A/B switches (environment): GMSB_KCLIQUE_M3NEED=4 builds a warp's third-level matrix only when at least
-            // four vertices are left to pick inside the set (default 3); GMSB_KCLIQUE_HUGE=old selects the round-1
-            // one-CTA-per-vertex-part kernel for d+ > 512 instead of the decoupled pair kernel
-            auto env_int = [](const char *name, int dflt) {
-                const char *e = std::getenv(name);
-                return e ? std::atoi(e) : dflt;
-            };
-            const int lane_flags = std::min(4, std::max(3, env_int("GMSB_KCLIQUE_M3NEED", 3))) << lane::kFlagM3NeedShift;
-            const char *huge_env = std::getenv("GMSB_KCLIQUE_HUGE");
-            // the pair kernel searches through third-level matrices, which pay when >= 5 vertices are left below (u, S[i]);
-            // GMSB_KCLIQUE_HUGE=pair forces it for smaller k (then it searches M2 directly with the flat lanes).
-            // GMSB_KCLIQUE_PAIR_MIN=512|256|128: smallest out-degree class that goes through the pair kernel.
-            const bool huge_old = huge_env ? !std::strcmp(huge_env, "old") : k < 7;
-            const int pair_min = env_int("GMSB_KCLIQUE_PAIR_MIN", kPairMinDefault);
-            const int64_t n_pair = huge_old ? 0 : (pair_min <= 128 ? bound[2] : (pair_min <= 256 ? bound[1] : bound[0]));
-            const int64_t mid_from = huge_old ? (int64_t)bound[0] : n_pair;     // first vertex left to the class kernels
-            DevBuf<lane::u64> spill;
-            // GMSB_KCLIQUE_TRACE=1: device time of every class launch on stderr (profiling aid)
-            const bool trace = std::getenv("GMSB_KCLIQUE_TRACE") != nullptr;
-            cudaEvent_t ev[6] = {};
-            unsigned long long seen[6] = {};
-            int nev = 0;
-            auto mark = [&]() {
-                if (!trace) return;
-                cudaEventCreate(&ev[nev]);
-                cudaEventRecord(ev[nev], r.stream);
-                seen[nev++] = total.get(0);          // synchronises: per-class counts for the trace
-            };
-            mark();
-            // The five class kernels are independent (own ticket, atomics on one total).  Each goes to its own stream
-            // so that the CTAs of the next class fill the SMs that the previous class's last items leave idle; with
-            // the sub-problems split over several GPUs those tails are a visible share of a launch.  (Serial when
-            // tracing, so that the per-class times mean something.)
-            struct AuxStreams {
-                cudaStream_t s[4] = {nullptr, nullptr, nullptr, nullptr};
-                cudaEvent_t ev = nullptr;
-                ~AuxStreams() {
-                    for (auto st : s) if (st) cudaStreamDestroy(st);
-                    if (ev) cudaEventDestroy(ev);
-                }
-            } auxs;
-            cudaStream_t (&aux)[4] = auxs.s;
-            cudaEvent_t &ready = auxs.ev;
-            if (!trace) {
-                GMSB_CUDA(cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
-                GMSB_CUDA(cudaEventRecord(ready, r.stream));
-                for (auto &st : aux) {
-                    GMSB_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-                    GMSB_CUDA(cudaStreamWaitEvent(st, ready, 0));
-                }
-            }
-            int next_aux = 0;
-            DevBuf<int64_t> pair_base, m1_off;
-            DevBuf<lane::u64> m1;
-            if (n_pair) {
-                // d+ > 512, decoupled: M1 of every such vertex to global memory, then (vertex, member) items.
-                // Sizes come from the (few thousand) out-degrees on the host; the vertices are processed in batches
-                // whose matrices fit kM1Budget bytes.
-                std::vector<vid_t> hv((size_t)n_pair);
-                GMSB_CUDA(cudaMemcpyAsync(hv.data(), vb.p, sizeof(vid_t) * n_pair, cudaMemcpyDeviceToHost, r.stream));
-                GMSB_CUDA(cudaStreamSynchronize(r.stream));
-                std::vector<int> hd((size_t)n_pair);
-                {
-                    // out-degrees of the listed vertices (descending): two offsets each
-                    DevBuf<int> dd((size_t)n_pair);
-                    k_list_degrees<<<grid_for(n_pair, 256), 256, 0, r.stream>>>(vb.p, n_pair, off, dd.p); launched();
-                    dd.download(hd.data(), (size_t)n_pair);
-                }
-                constexpr size_t kM1Budget = size_t(12) << 30;
-                constexpr int PBLOCK = 256;
-                const size_t smem2 = lane::pair_smem_words(maxD, PBLOCK / 32) * 8;
-                GMSB_REQUIRE(smem2 + 4096 <= r.smem_optin, "kclique_count: out-degree too large for the pair kernel");
-                auto kern2 = lane::k_kclique_lane_pair<PBLOCK>;
-                GMSB_CUDA(cudaFuncSetAttribute(kern2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-                int resident2 = 0;
-                GMSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident2, kern2, PBLOCK, smem2));
-                GMSB_REQUIRE(resident2 >= 1, "kclique_count: pair kernel does not fit on an SM");
-                constexpr int BBLOCK = 256;
-                const size_t smem1 = ((size_t)(BBLOCK / 32) * lane::huge_pitch(maxD) + (size_t)((maxD + 1) >> 1)) * 8;
-                auto kern1 = lane::k_kclique_m1_build<BBLOCK>;
-                GMSB_CUDA(cudaFuncSetAttribute(kern1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-                int64_t t0 = 0;
-                int64_t item0 = 0;                       // global numbering of the items, for the multi-GPU deal
-                while (t0 < n_pair) {
-                    std::vector<int64_t> h_m1((size_t)0), h_items((size_t)0);
-                    size_t words = 0;
-                    int64_t items = 0, t1 = t0;
-                    while (t1 < n_pair) {
-                        const size_t w = (size_t)hd[t1] * (size_t)lane::huge_pitch(hd[t1]);
-                        if (t1 > t0 && (words + w) * 8 > kM1Budget) break;
-                        h_m1.push_back((int64_t)words); h_items.push_back(items);
-                        words += w; items += hd[t1]; ++t1;
-                    }
-                    h_items.push_back(items);
-                    const int64_t nv = t1 - t0;
-                    m1.alloc(words);
-                    m1_off.alloc((size_t)nv); pair_base.alloc((size_t)nv + 1);
-                    m1_off.upload(h_m1.data(), (size_t)nv);
-                    pair_base.upload(h_items.data(), (size_t)nv + 1);
-                    const int grid1 = (int)std::min<int64_t>(nv, (int64_t)r.sm_count * 4);
-                    kern1<<<grid1, BBLOCK, smem1, r.stream>>>(vb.p, t0, nv, off, nbr, m1_off.p, m1.p, maxD); launched();
-                    // this process's items of the batch: global item numbers congruent to pi modulo P
-                    const int shift = (int)(((int64_t)pi - item0 % P + P) % P);
-                    const int64_t mine = items > shift ? (items - shift + P - 1) / P : 0;
-                    if (mine) {
-                        GMSB_CUDA(cudaMemsetAsync(tickets.p, 0, sizeof(unsigned int), r.stream));
-                        const int grid2 = (int)std::min<int64_t>(mine, (int64_t)r.sm_count * resident2);
-                        kern2<<<grid2, PBLOCK, smem2, r.stream>>>(vb.p, t0, pair_base.p, nv, items, off, m1_off.p, m1.p, k,
-                                                                  maxD, total.p, tickets.p, shift, P, lane_flags);
-                        launched();
-                    }
-                    GMSB_CUDA(cudaStreamSynchronize(r.stream));      // host vectors / batch buffers are reused
-                    item0 += items;
-                    t0 = t1;
-                }
-            } else if (n_huge && huge_old) {    // round-1 kernel: CTA-wide top of the tree, compact matrices below, one CTA per SM
-                exclusive_sum(parts.p, item_base.p, n_huge + 1);
-                const int64_t n_items = item_base.get(n_huge);
-                auto launch_huge = [&](auto kern, int block) {
-                    const size_t full = lane::huge_smem_words(maxD, true) * 8;
-                    const bool in_smem = full + 2048 <= r.smem_optin;
-                    const size_t smem = in_smem ? full : lane::huge_smem_words(maxD, false) * 8;
-                    GMSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                    const int grid = (int)std::min<int64_t>(n_items, (int64_t)r.sm_count);
-                    if (!in_smem) spill.alloc((size_t)grid * (size_t)maxD * (size_t)lane::huge_pitch(maxD));
-                    kern<<<grid, block, smem, r.stream>>>(vb.p, item_base.p, n_huge, n_items, off, nbr, k, maxD, total.p,
-                                                          tickets.p, in_smem ? nullptr : spill.p, pi, P);
-                    launched();
-                };
-                // 512 threads cap the kernel at 128 registers and it spills; 384 threads (168 registers, no spills) were
-                // 6 % faster at scale 22, k = 6.  GMSB_KCLIQUE_HUGE_BLOCK=512 selects the other build for A/B runs.
-                const char *hb = std::getenv("GMSB_KCLIQUE_HUGE_BLOCK");
-                if (hb && std::atoi(hb) == 512) launch_huge(lane::k_kclique_lane_huge<512>, 512);
-                else launch_huge(lane::k_kclique_lane_huge<384>, 384);
-            }
-            mark();
-            // third-level boxes only where they shorten the rows: matrices of 4 or 8 words per row
-            auto mid = [&](auto kern, int block, bool boxes, int64_t first, int64_t cnt, unsigned int *ticket) {
-                if (cnt <= 0) return;
-                const int flags = lane_flags;
-                const size_t dyn = boxes ? (size_t)(block / 32) * sizeof(lane::WarpBox) : 0;
-                GMSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-                int resident = 0;
-                GMSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, block, dyn));
-                GMSB_REQUIRE(resident >= 1, "kclique_count: kernel does not fit on an SM");
-                const int grid = (int)std::min<int64_t>(cnt, (int64_t)r.sm_count * resident);
-                cudaStream_t st = trace ? r.stream : aux[next_aux++];
-                kern<<<grid, block, dyn, st>>>(vb.p + first, cnt, off, nbr, k, total.p, ticket, pi, P, flags);
-                launched();
-            };
-            auto mid_marked = [&](auto kern, int block, bool boxes, int64_t first, int64_t cnt, unsigned int *ticket) {
-                mid(kern, block, boxes, first, cnt, ticket);
-                mark();
-            };
-            auto from = [&](int64_t b) { return std::max<int64_t>(b, mid_from); };
-            mid_marked(lane::k_kclique_lane_mid<8, 384, 2>, 384, true, from(bound[0]), bound[1] - from(bound[0]), tickets.p + 1);
-            mid_marked(lane::k_kclique_lane_mid<4, 256, 4>, 256, true, from(bound[1]), bound[2] - from(bound[1]), tickets.p + 2);
-            mid_marked(lane::k_kclique_lane_mid<2, 128, 8>, 128, false, from(bound[2]), bound[3] - from(bound[2]), tickets.p + 3);
-            mid_marked(lane::k_kclique_lane_mid<1, 128, 8>, 128, false, bound[3], nb - bound[3], tickets.p + 4);
-            if (!trace) {
-                for (auto &st : aux) {           // join: the library stream continues after every class
-                    GMSB_CUDA(cudaEventRecord(ready, st));
-                    GMSB_CUDA(cudaStreamWaitEvent(r.stream, ready, 0));
-                }
-            }
-            GMSB_CUDA(cudaStreamSynchronize(r.stream));
-            if (trace) {
-                static const char *names[5] = {"huge(d+>512)", "mid8(<=512)", "mid4(<=256)", "mid2(<=128)", "mid1(<=64)"};
-                const int64_t counts[5] = {n_huge, bound[1] - bound[0], bound[2] - bound[1], bound[3] - bound[2],
-                                           nb - bound[3]};
-                for (int i = 0; i + 1 < nev; ++i) {
-                    float ms = 0;
-                    cudaEventElapsedTime(&ms, ev[i], ev[i + 1]);
-                    std::fprintf(stderr, "[gmsb kclique k=%d] %-13s vertices=%lld ms=%.3f cliques=%llu\n", k, names[i],
-                                 (long long)counts[i], ms, seen[i + 1] - seen[i]);
-                }
-                for (int i = 0; i < nev; ++i) cudaEventDestroy(ev[i]);
-            }
-        } else {
-            run_class(0, n_huge, maxD, true);
-            run_class(n_huge, nb - n_huge, kMidD, false);
-        }
+        DevBuf<int> cc(4);
+        cc.zero();
+        k_class_counts<<<grid_for(nb, 256), 256, 0, r.stream>>>(vb.p, nb, off, cc.p); launched();
+        int bound[4];
+        cc.download(bound, 4);
+        const BigVerts b{vb.p, nb, {bound[0], bound[1], bound[2], bound[3]}, maxD, off, nbr, k, pi, P, total};
+        // lane-parallel kernels where they are faster (B200 measurements, DESIGN.md §3.4) and their path register
+        // holds the search (k - 1 <= lane::kMaxNeed); warp-cooperative otherwise
+        if (k < 5 || k - 1 > lane::kMaxNeed) count_warp(b);
+        else if (k < 7) count_lane_huge(b);
+        else count_lane_pair(b);
     }
     return total.get(0);
 }

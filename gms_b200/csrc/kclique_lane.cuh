@@ -113,9 +113,6 @@ __device__ __forceinline__ u64 lane_tasks_flat(const u64 *cm, int pitch, unsigne
     return total;
 }
 
-// flags of the lane kernels (kernel argument, set by kclique.cu from the environment for A/B runs)
-constexpr int kFlagM3NeedShift = 4;    // bits 4..7: smallest number of vertices left for which a warp builds an M3 (3 or 4)
-
 // ---- third level: per-warp compact matrix ------------------------------------------------------------------------------
 // Deep in the tree the candidate sets hold 3-5 members per 64-bit word of the parent's index space, so every AND +
 // popcount there is mostly zeros.  A WARP therefore re-indexes a candidate set of <= kC3Max = 192 members into a
@@ -162,8 +159,7 @@ __device__ __forceinline__ u64 lane_triangles_in_set(const u64 *cm, int pitch, i
 
 // `need`-cliques (need >= 1) among the members of box->sets[level0] (nw valid words, the rest zero), by the whole warp.
 // Returns this lane's partial count.
-__device__ __forceinline__ u64 warp_set_count(const u64 *cm, int pitch, int nw, WarpBox *box, int level0, int need0, int lane,
-                                              int flags) {
+__device__ __forceinline__ u64 warp_set_count(const u64 *cm, int pitch, int nw, WarpBox *box, int level0, int need0, int lane) {
     u64 total = 0;
     int level = level0, need = need0;
     bool fresh = true;
@@ -264,7 +260,7 @@ __device__ __forceinline__ u64 warp_set_count(const u64 *cm, int pitch, int nw, 
 // by all lanes of the CTA, 64 residue-class tasks per row.
 template <int NWP, bool FLATBIG>
 __device__ __forceinline__ u64 count_compact_boxes(const u64 *cm, int pitch, int nw, int c, int need, unsigned *counter,
-                                                   WarpBox *box, CtaBigRows *big, int lane, int flags) {
+                                                   WarpBox *box, CtaBigRows *big, int lane) {
     u64 total = 0;
     for (;;) {
         unsigned a = 0;
@@ -285,7 +281,7 @@ __device__ __forceinline__ u64 count_compact_boxes(const u64 *cm, int pitch, int
         __syncwarp();
         if (lane < 8) box->sets[0][lane] = mine;
         __syncwarp();
-        total += warp_set_count(cm, pitch, nw, box, 0, need - 1, lane, flags);
+        total += warp_set_count(cm, pitch, nw, box, 0, need - 1, lane);
     }
     __syncthreads();
     const unsigned t_end = big->count << 6;
@@ -300,9 +296,9 @@ __device__ __forceinline__ u64 count_compact_boxes(const u64 *cm, int pitch, int
 // one per (k-1)-clique: it pays for d <= k - 4, i.e. need >= 5 here); else per-lane tasks over every member.
 template <int NW>
 __device__ __forceinline__ u64 count_compact(const u64 *cm, int pitch, int c, int need, int block, unsigned *counter,
-                                             WarpBox *box, CtaBigRows *big, int lane, int flags) {
+                                             WarpBox *box, CtaBigRows *big, int lane) {
     if constexpr (NW >= 3) {
-        if (box && need >= 5) return count_compact_boxes<NW, false>(cm, pitch, NW, c, need, counter, box, big, lane, flags);
+        if (box && need >= 5) return count_compact_boxes<NW, false>(cm, pitch, NW, c, need, counter, box, big, lane);
     }
     const int sl = split_for(c, block);
     if constexpr (NW <= 2) return lane_tasks_flat<NW>(cm, pitch, (unsigned)c << sl, need, sl, counter, lane, nullptr);
@@ -336,7 +332,7 @@ template <int NWB, int BLOCK, int MINB>
 __global__ void __launch_bounds__(BLOCK, MINB)
 k_kclique_lane_mid(const vid_t *__restrict__ verts, int64_t count, const eid_t *__restrict__ off,
                    const vid_t *__restrict__ nbr, int k, unsigned long long *__restrict__ total,
-                   unsigned int *__restrict__ ticket, int pi, int P, int flags) {
+                   unsigned int *__restrict__ ticket, int pi, int P) {
     constexpr int DMAX = 64 * NWB;
     constexpr int PITCH = pitch_for(NWB);
     __shared__ vid_t S[DMAX];
@@ -363,7 +359,7 @@ k_kclique_lane_mid(const vid_t *__restrict__ verts, int64_t count, const eid_t *
         build_rows<BLOCK>(S, D, M, PITCH, off, nbr, tid);
         __syncthreads();
         // u is the first clique vertex; k-1 more inside the matrix
-        acc += count_compact<NWB>(M, PITCH, D, k - 1, BLOCK, &s_counter, box, &s_big, lane, flags);
+        acc += count_compact<NWB>(M, PITCH, D, k - 1, BLOCK, &s_counter, box, &s_big, lane);
     }
     const unsigned long long s = block_sum(acc, red);
     if (tid == 0 && s) atomicAdd(total, s);
@@ -378,6 +374,131 @@ __host__ __device__ inline size_t huge_smem_words(int maxD, bool matrix_in_smem)
     const size_t P1 = (size_t)huge_pitch(maxD);
     return (matrix_in_smem ? (size_t)maxD * P1 : 0) + (size_t)kCMax * pitch_for(8) + (size_t)kStackLevels * P1 +
            (size_t)((maxD + 1) >> 1) + ((P1 + 2) >> 1) + (size_t)(kCMax / 4);
+}
+
+// index t of the vertex that work item `item` belongs to: item_base[t] <= item < item_base[t + 1] (item_base is the
+// exclusive scan of the items per vertex, nverts + 1 entries)
+__device__ __forceinline__ int64_t item_vertex(const int64_t *item_base, int64_t nverts, int64_t item) {
+    int64_t lo_t = 0, hi_t = nverts;
+    while (hi_t - lo_t > 1) {
+        const int64_t mid = (lo_t + hi_t) >> 1;
+        if (item_base[mid] <= item) lo_t = mid; else hi_t = mid;
+    }
+    return lo_t;
+}
+
+// The CTA walks the top of the search tree below u and S[i] together (k_kclique_lane_huge, k_kclique_lane_pair).
+// M1 is the bit matrix of S (|S| = D, W1 valid words per row, pitch P1); stack[level] = candidates after (level + 2)
+// chosen vertices, and the caller has written stack[0] = row i of M1 and passed a barrier.  A set with one or two
+// vertices left is counted straight off M1; one of <= kCMax members is re-indexed into the compact matrix M2 and
+// counted by the kernel's own step; a larger set is expanded one member at a time.  What differs between the kernels:
+//   PAD                 rows of M2 are zero padded from 3..8 words to 4 or 8 (else exactly nwb words);
+//   reset()             thread 0, before the barrier that precedes M2: zero the kernel's tickets;
+//   count(M2, pitch2, nwb, nwp, c, need, acc)   all threads: acc plus this thread's share of the need-cliques of M2
+//                       (c members, nwb valid words per row, nwp readable).
+// All threads of the CTA must be here.  Returns acc plus this thread's partial count.
+template <int BLOCK, bool PAD, class Reset, class Count>
+__device__ __forceinline__ u64 cta_walk(const u64 *M1, int P1, int W1, int D, int k, u64 *stack, u64 *M2, int *prefix,
+                                        unsigned short *list, int &s_c, const Reset &reset, const Count &count, u64 acc) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    int level = 0;
+    bool fresh = true;
+    int cursor[kStackLevels];
+    for (;;) {
+        const u64 *set = stack + (size_t)level * P1;
+        if (fresh) {
+            fresh = false;
+            if (warp == 0) {
+                int pc = 0;
+                for (int w = lane; w < W1; w += 32) pc += __popcll(set[w]);
+                for (int o = 16; o; o >>= 1) pc += __shfl_xor_sync(0xffffffffu, pc, o);
+                if (lane == 0) s_c = pc;
+            }
+            __syncthreads();
+            const int c = s_c;
+            const int need = k - level - 2;
+            bool expand = false;
+            if (c >= need) {
+                if (need == 1) {
+                    if (tid == 0) acc += (u64)c;
+                } else if (need == 2) {
+                    // pairs straight off the big matrix: thread per member
+                    unsigned cnt = 0;
+                    for (int p = tid; p < D; p += BLOCK) {
+                        const int w0 = p >> 6;
+                        if ((set[w0] >> (p & 63)) & 1ull) {
+                            const u64 *row = M1 + (size_t)p * P1;
+                            for (int w = w0; w < W1; ++w) cnt += (unsigned)__popcll(set[w] & row[w]);
+                        }
+                    }
+                    acc += cnt;
+                } else if (c <= kCMax) {
+                    // re-index the set into the compact matrix and deal its subtrees to the lanes
+                    if (warp == 0) {
+                        int carry = 0;
+                        for (int base = 0; base < P1; base += 32) {
+                            const int w = base + lane;
+                            const int v = w < W1 ? __popcll(set[w]) : 0;
+                            int incl = v;
+                            for (int o = 1; o < 32; o <<= 1) {
+                                const int x = __shfl_up_sync(0xffffffffu, incl, o);
+                                if (lane >= o) incl += x;
+                            }
+                            if (w < P1) prefix[w] = carry + incl - v;
+                            carry += __shfl_sync(0xffffffffu, incl, 31);
+                        }
+                    }
+                    if (tid == 0) reset();
+                    __syncthreads();
+                    for (int p = tid; p < D; p += BLOCK)
+                        if ((set[p >> 6] >> (p & 63)) & 1ull)
+                            list[compact_index(set, prefix, p)] = (unsigned short)p;
+                    __syncthreads();
+                    const int nwb = (c + 63) >> 6;         // 1..8 words per compact row
+                    const int nwp = PAD ? (nwb <= 2 ? nwb : (nwb <= 4 ? 4 : 8)) : nwb;
+                    const int pitch2 = pitch_for(nwp);
+                    for (int a = tid; a < c; a += BLOCK) {
+                        const int pa = list[a];
+                        compact_row(set, prefix, W1, M1 + (size_t)pa * P1, pa, M2 + (size_t)a * pitch2, nwp);
+                    }
+                    __syncthreads();
+                    acc = count(M2, pitch2, nwb, nwp, c, need, acc);
+                } else {
+                    expand = true;
+                }
+            }
+            if (!expand) {
+                if (level == 0) break;
+                --level;
+                continue;
+            }
+            cursor[level] = -1;
+        }
+        // next member of this level's set after the cursor (every thread computes the same answer)
+        int v = -1;
+        {
+            const int from = cursor[level] + 1;
+            int w = from >> 6;
+            if (w < W1) {
+                u64 m = set[w] & (~0ull << (from & 63));
+                while (!m && ++w < W1) m = set[w];
+                if (m) v = (w << 6) + __ffsll((long long)m) - 1;
+            }
+        }
+        if (v < 0) {
+            if (level == 0) break;
+            --level;
+            continue;
+        }
+        cursor[level] = v;
+        __syncthreads();          // everyone is done with the deeper levels before they are overwritten
+        u64 *child = stack + (size_t)(level + 1) * P1;
+        for (int w = tid; w < P1; w += BLOCK) child[w] = set[w] & M1[(size_t)v * P1 + w];
+        __syncthreads();
+        ++level;
+        fresh = true;
+    }
+    return acc;
 }
 
 template <int BLOCK>
@@ -398,7 +519,23 @@ k_kclique_lane_huge(const vid_t *__restrict__ verts, const int64_t *__restrict__
     __shared__ unsigned long long red[BLOCK / 32];
     __shared__ unsigned int s_item, s_counter;
     __shared__ int s_c;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x, lane = tid & 31;
+    // compact step: rows of exactly nwb words, per-lane tasks over every member
+    auto reset = [&] { s_counter = 0; };
+    auto count_m2 = [&](const u64 *M2, int pitch2, int nwb, int, int c, int need, u64 acc) {
+        const int sl = split_for(c, BLOCK);
+        switch (nwb) {
+            case 1: acc += lane_tasks<1>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
+            case 2: acc += lane_tasks<2>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
+            case 3: acc += lane_tasks<3>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
+            case 4: acc += lane_tasks<4>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
+            case 5: acc += lane_tasks<5>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
+            case 6: acc += lane_tasks<6>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
+            case 7: acc += lane_tasks<7>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
+            default: acc += lane_tasks<8>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
+        }
+        return acc;
+    };
     u64 acc = 0;
     for (;;) {
         __syncthreads();
@@ -406,12 +543,7 @@ k_kclique_lane_huge(const vid_t *__restrict__ verts, const int64_t *__restrict__
         __syncthreads();
         const int64_t item = pi + (int64_t)s_item * P;
         if (item >= count) break;
-        int64_t lo_t = 0, hi_t = nverts;
-        while (hi_t - lo_t > 1) {
-            const int64_t mid = (lo_t + hi_t) >> 1;
-            if (item_base[mid] <= item) lo_t = mid; else hi_t = mid;
-        }
-        const int64_t t = lo_t;
+        const int64_t t = item_vertex(item_base, nverts, item);
         const int part = (int)(item - item_base[t]), nparts = (int)(item_base[t + 1] - item_base[t]);
         const vid_t u = verts[t];
         const eid_t ob = off[u];
@@ -421,117 +553,11 @@ k_kclique_lane_huge(const vid_t *__restrict__ verts, const int64_t *__restrict__
         for (size_t j = tid; j < (size_t)D * P1; j += BLOCK) M1[j] = 0ull;
         __syncthreads();
         build_rows<BLOCK>(S, D, M1, P1, off, nbr, tid);
-        // the CTA walks the top of the tree together: stack[level] = candidates after (level + 2) chosen vertices
         for (int i = part; i < D; i += nparts) {
             __syncthreads();
             for (int w = tid; w < P1; w += BLOCK) stack[w] = M1[(size_t)i * P1 + w];
             __syncthreads();
-            int level = 0;
-            bool fresh = true;
-            int cursor[kStackLevels];
-            for (;;) {
-                const u64 *set = stack + (size_t)level * P1;
-                if (fresh) {
-                    fresh = false;
-                    if (warp == 0) {
-                        int pc = 0;
-                        for (int w = lane; w < W1; w += 32) pc += __popcll(set[w]);
-                        for (int o = 16; o; o >>= 1) pc += __shfl_xor_sync(0xffffffffu, pc, o);
-                        if (lane == 0) s_c = pc;
-                    }
-                    __syncthreads();
-                    const int c = s_c;
-                    const int need = k - level - 2;
-                    bool expand = false;
-                    if (c >= need) {
-                        if (need == 1) {
-                            if (tid == 0) acc += (u64)c;
-                        } else if (need == 2) {
-                            // pairs straight off the big matrix: thread per member
-                            unsigned cnt = 0;
-                            for (int p = tid; p < D; p += BLOCK) {
-                                const int w0 = p >> 6;
-                                if ((set[w0] >> (p & 63)) & 1ull) {
-                                    const u64 *row = M1 + (size_t)p * P1;
-                                    for (int w = w0; w < W1; ++w) cnt += (unsigned)__popcll(set[w] & row[w]);
-                                }
-                            }
-                            acc += cnt;
-                        } else if (c <= kCMax) {
-                            // re-index the set into the compact matrix and deal its subtrees to the lanes
-                            if (warp == 0) {
-                                int carry = 0;
-                                for (int base = 0; base < P1; base += 32) {
-                                    const int w = base + lane;
-                                    const int v = w < W1 ? __popcll(set[w]) : 0;
-                                    int incl = v;
-                                    for (int o = 1; o < 32; o <<= 1) {
-                                        const int x = __shfl_up_sync(0xffffffffu, incl, o);
-                                        if (lane >= o) incl += x;
-                                    }
-                                    if (w < P1) prefix[w] = carry + incl - v;
-                                    carry += __shfl_sync(0xffffffffu, incl, 31);
-                                }
-                            }
-                            if (tid == 0) s_counter = 0;
-                            __syncthreads();
-                            for (int p = tid; p < D; p += BLOCK)
-                                if ((set[p >> 6] >> (p & 63)) & 1ull)
-                                    list[compact_index(set, prefix, p)] = (unsigned short)p;
-                            __syncthreads();
-                            const int nwb = (c + 63) >> 6;         // 1..8 words per compact row
-                            const int pitch2 = pitch_for(nwb);
-                            for (int a = tid; a < c; a += BLOCK) {
-                                const int pa = list[a];
-                                compact_row(set, prefix, W1, M1 + (size_t)pa * P1, pa, M2 + (size_t)a * pitch2, nwb);
-                            }
-                            __syncthreads();
-                            const int sl = split_for(c, BLOCK);
-                            switch (nwb) {
-                                case 1: acc += lane_tasks<1>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
-                                case 2: acc += lane_tasks<2>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
-                                case 3: acc += lane_tasks<3>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
-                                case 4: acc += lane_tasks<4>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
-                                case 5: acc += lane_tasks<5>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
-                                case 6: acc += lane_tasks<6>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
-                                case 7: acc += lane_tasks<7>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
-                                default: acc += lane_tasks<8>(M2, pitch2, (unsigned)c << sl, need, sl, &s_counter, lane, nullptr); break;
-                            }
-                        } else {
-                            expand = true;
-                        }
-                    }
-                    if (!expand) {
-                        if (level == 0) break;
-                        --level;
-                        continue;
-                    }
-                    cursor[level] = -1;
-                }
-                // next member of this level's set after the cursor (every thread computes the same answer)
-                int v = -1;
-                {
-                    const int from = cursor[level] + 1;
-                    int w = from >> 6;
-                    if (w < W1) {
-                        u64 m = set[w] & (~0ull << (from & 63));
-                        while (!m && ++w < W1) m = set[w];
-                        if (m) v = (w << 6) + __ffsll((long long)m) - 1;
-                    }
-                }
-                if (v < 0) {
-                    if (level == 0) break;
-                    --level;
-                    continue;
-                }
-                cursor[level] = v;
-                __syncthreads();          // everyone is done with the deeper levels before they are overwritten
-                u64 *child = stack + (size_t)(level + 1) * P1;
-                for (int w = tid; w < P1; w += BLOCK) child[w] = set[w] & M1[(size_t)v * P1 + w];
-                __syncthreads();
-                ++level;
-                fresh = true;
-            }
+            acc = cta_walk<BLOCK, false>(M1, P1, W1, D, k, stack, M2, prefix, list, s_c, reset, count_m2, acc);
         }
     }
     const unsigned long long s = block_sum(acc, red);
@@ -541,14 +567,14 @@ k_kclique_lane_huge(const vid_t *__restrict__ verts, const int64_t *__restrict__
 // ---- d+ > 512, decoupled (round 2) -------------------------------------------------------------------------------------
 // k_kclique_lane_huge keeps the vertex's big matrix M1 in shared memory (up to 142 KB at scale 22), which leaves room
 // for one CTA per SM and nothing for per-warp third-level matrices.  Here the two jobs are separated:
-//   phase 1  k_kclique_m1_build   M1 of every d+ > 512 vertex is written to global memory (0.5 GB at scale 22; the
+//   phase 1  k_kclique_m1_build   M1 of every d+ > 128 vertex is written to global memory (0.5 GB at scale 22; the
 //                                 rows a CTA needs stay in the L2);
 //   phase 2  k_kclique_lane_pair  (k >= 7: at least five vertices left below u and S[i], so that third-level matrices
 //                                 pay) work item = (vertex u, member i): the CTA reads row i of M1 — the candidates after
 //                                 choosing u and S[i] —, walks further down together only while that set has more than
 //                                 512 members, re-indexes it into a compact matrix M2 in shared memory and counts in
 //                                 M2 exactly as the 257..512 class does (count_compact: per-warp M3 boxes, flat lanes).
-// Shared memory per CTA is M2 + boxes (~105 KB at 384 threads): two CTAs per SM, items ~100x finer than a vertex
+// Shared memory per CTA is M2 + boxes (~85 KB at 256 threads): two CTAs per SM, items ~100x finer than a vertex
 // part, and no limit on d+ other than the memory for M1.
 __host__ __device__ inline size_t pair_smem_words(int maxD, int warps) {
     const size_t P1 = (size_t)huge_pitch(maxD);
@@ -604,7 +630,7 @@ __global__ void __launch_bounds__(BLOCK, 2)
 k_kclique_lane_pair(const vid_t *__restrict__ verts, int64_t first, const int64_t *__restrict__ item_base,
                     int64_t nverts, int64_t count, const eid_t *__restrict__ off, const int64_t *__restrict__ m1_off,
                     const u64 *__restrict__ m1, int k, int maxD, unsigned long long *__restrict__ total,
-                    unsigned int *__restrict__ ticket, int pi, int P, int flags) {
+                    unsigned int *__restrict__ ticket, int pi, int P) {
     extern __shared__ u64 smem64[];
     const int P1max = huge_pitch(maxD);
     u64 *sp = smem64;
@@ -618,6 +644,26 @@ k_kclique_lane_pair(const vid_t *__restrict__ verts, int64_t first, const int64_
     __shared__ CtaBigRows s_big;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     WarpBox *box = reinterpret_cast<WarpBox *>(sp) + warp;
+    // compact step: rows padded to 4 or 8 words; per-warp M3 boxes where five or more vertices are left, else flat lanes
+    auto reset = [&] { s_counter = 0; s_big.count = 0; s_big.counter = 0; };
+    auto count_m2 = [&](const u64 *M2, int pitch2, int nwb, int nwp, int c, int need, u64 acc) {
+        if (nwp == 8 && need >= 5) {
+            acc += count_compact_boxes<8, true>(M2, pitch2, nwb, c, need, &s_counter, box, &s_big, lane);
+        } else if (nwp == 4 && need >= 5) {
+            acc += count_compact_boxes<4, true>(M2, pitch2, nwb, c, need, &s_counter, box, &s_big, lane);
+        } else if (nwp >= 4) {       // too shallow for another re-indexing: flat lanes on M2 itself
+            const int sl = split_for(c, BLOCK);
+            const unsigned t_end = (unsigned)c << sl;
+            acc += nwp == 4 ? lane_tasks_flat<4>(M2, pitch2, t_end, need, sl, &s_counter, lane, nullptr)
+                            : lane_tasks_flat<8>(M2, pitch2, t_end, need, sl, &s_counter, lane, nullptr);
+        } else {
+            const int sl = split_for(c, BLOCK);
+            const unsigned t_end = (unsigned)c << sl;
+            acc += nwb == 1 ? lane_tasks_flat<1>(M2, pitch2, t_end, need, sl, &s_counter, lane, nullptr)
+                            : lane_tasks_flat<2>(M2, pitch2, t_end, need, sl, &s_counter, lane, nullptr);
+        }
+        return acc;
+    };
     u64 acc = 0;
     for (;;) {
         __syncthreads();
@@ -625,12 +671,7 @@ k_kclique_lane_pair(const vid_t *__restrict__ verts, int64_t first, const int64_
         __syncthreads();
         const int64_t item = pi + (int64_t)s_item * P;
         if (item >= count) break;
-        int64_t lo_t = 0, hi_t = nverts;
-        while (hi_t - lo_t > 1) {
-            const int64_t mid = (lo_t + hi_t) >> 1;
-            if (item_base[mid] <= item) lo_t = mid; else hi_t = mid;
-        }
-        const int64_t t = lo_t;
+        const int64_t t = item_vertex(item_base, nverts, item);
         const int i = (int)(item - item_base[t]);
         const vid_t u = verts[first + t];
         const int D = (int)(off[u + 1] - off[u]);
@@ -638,115 +679,8 @@ k_kclique_lane_pair(const vid_t *__restrict__ verts, int64_t first, const int64_
         const u64 *__restrict__ M1 = m1 + m1_off[t];
         for (int w = tid; w < P1; w += BLOCK) stack[w] = M1[(size_t)i * P1 + w];
         __syncthreads();
-        // stack[level] = candidates after (level + 2) chosen vertices; the CTA walks down together while they are > 512
-        int level = 0;
-        bool fresh = true;
-        int cursor[kStackLevels];
-        for (;;) {
-            const u64 *set = stack + (size_t)level * P1;
-            if (fresh) {
-                fresh = false;
-                if (warp == 0) {
-                    int pc = 0;
-                    for (int w = lane; w < W1; w += 32) pc += __popcll(set[w]);
-                    for (int o = 16; o; o >>= 1) pc += __shfl_xor_sync(0xffffffffu, pc, o);
-                    if (lane == 0) s_c = pc;
-                }
-                __syncthreads();
-                const int c = s_c;
-                const int need = k - level - 2;
-                bool expand = false;
-                if (c >= need) {
-                    if (need == 1) {
-                        if (tid == 0) acc += (u64)c;
-                    } else if (need == 2) {
-                        unsigned cnt = 0;
-                        for (int p = tid; p < D; p += BLOCK) {
-                            const int w0 = p >> 6;
-                            if ((set[w0] >> (p & 63)) & 1ull) {
-                                const u64 *row = M1 + (size_t)p * P1;
-                                for (int w = w0; w < W1; ++w) cnt += (unsigned)__popcll(set[w] & row[w]);
-                            }
-                        }
-                        acc += cnt;
-                    } else if (c <= kCMax) {
-                        if (warp == 0) {
-                            int carry = 0;
-                            for (int base = 0; base < P1; base += 32) {
-                                const int w = base + lane;
-                                const int v = w < W1 ? __popcll(set[w]) : 0;
-                                int incl = v;
-                                for (int o = 1; o < 32; o <<= 1) {
-                                    const int x = __shfl_up_sync(0xffffffffu, incl, o);
-                                    if (lane >= o) incl += x;
-                                }
-                                if (w < P1) prefix[w] = carry + incl - v;
-                                carry += __shfl_sync(0xffffffffu, incl, 31);
-                            }
-                        }
-                        if (tid == 0) { s_counter = 0; s_big.count = 0; s_big.counter = 0; }
-                        __syncthreads();
-                        for (int p = tid; p < D; p += BLOCK)
-                            if ((set[p >> 6] >> (p & 63)) & 1ull)
-                                list[compact_index(set, prefix, p)] = (unsigned short)p;
-                        __syncthreads();
-                        const int nwb = (c + 63) >> 6;         // 1..8 words per compact row ...
-                        const int nwp = nwb <= 2 ? nwb : (nwb <= 4 ? 4 : 8);     // ... zero padded to 4 or 8
-                        const int pitch2 = pitch_for(nwp);
-                        for (int a = tid; a < c; a += BLOCK) {
-                            const int pa = list[a];
-                            compact_row(set, prefix, W1, M1 + (size_t)pa * P1, pa, M2 + (size_t)a * pitch2, nwp);
-                        }
-                        __syncthreads();
-                        if (nwp == 8 && need >= 5) {
-                            acc += count_compact_boxes<8, true>(M2, pitch2, nwb, c, need, &s_counter, box, &s_big, lane, flags);
-                        } else if (nwp == 4 && need >= 5) {
-                            acc += count_compact_boxes<4, true>(M2, pitch2, nwb, c, need, &s_counter, box, &s_big, lane, flags);
-                        } else if (nwp >= 4) {       // too shallow for another re-indexing: flat lanes on M2 itself
-                            const int sl = split_for(c, BLOCK);
-                            const unsigned t_end = (unsigned)c << sl;
-                            acc += nwp == 4 ? lane_tasks_flat<4>(M2, pitch2, t_end, need, sl, &s_counter, lane, nullptr)
-                                            : lane_tasks_flat<8>(M2, pitch2, t_end, need, sl, &s_counter, lane, nullptr);
-                        } else {
-                            const int sl = split_for(c, BLOCK);
-                            const unsigned t_end = (unsigned)c << sl;
-                            acc += nwb == 1 ? lane_tasks_flat<1>(M2, pitch2, t_end, need, sl, &s_counter, lane, nullptr)
-                                            : lane_tasks_flat<2>(M2, pitch2, t_end, need, sl, &s_counter, lane, nullptr);
-                        }
-                    } else {
-                        expand = true;
-                    }
-                }
-                if (!expand) {
-                    if (level == 0) break;
-                    --level;
-                    continue;
-                }
-                cursor[level] = -1;
-            }
-            int v = -1;
-            {
-                const int from = cursor[level] + 1;
-                int w = from >> 6;
-                if (w < W1) {
-                    u64 m = set[w] & (~0ull << (from & 63));
-                    while (!m && ++w < W1) m = set[w];
-                    if (m) v = (w << 6) + __ffsll((long long)m) - 1;
-                }
-            }
-            if (v < 0) {
-                if (level == 0) break;
-                --level;
-                continue;
-            }
-            cursor[level] = v;
-            __syncthreads();          // everyone is done with the deeper levels before they are overwritten
-            u64 *child = stack + (size_t)(level + 1) * P1;
-            for (int w = tid; w < P1; w += BLOCK) child[w] = set[w] & M1[(size_t)v * P1 + w];
-            __syncthreads();
-            ++level;
-            fresh = true;
-        }
+        // the CTA walks down together while the candidate set has more than 512 members
+        acc = cta_walk<BLOCK, true>(M1, P1, W1, D, k, stack, M2, prefix, list, s_c, reset, count_m2, acc);
     }
     const unsigned long long s = block_sum(acc, red);
     if (tid == 0 && s) atomicAdd(total, s);

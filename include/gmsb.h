@@ -281,8 +281,8 @@ GMSB_API int gmsb_edge_similarity(gmsb_graph_t g, int metric, double *out, int64
 /* KClique::Par::{NP,EP}_kclisting on an oriented DAG      gms/algorithms/non_set_based/k_clique_list/clique_counting.h:14-34
  * g may be a DAG from gmsb_orient, or an undirected graph (then it is degree-oriented internally; the count is
  * orientation-invariant). k==1 -> nodes, k==2 -> edges as parallelize.h:43-44.
- * Kernel family for the d+ > 32 sub-problems: lane-parallel (5 <= k <= 10) or warp-cooperative (otherwise); the
- * environment variable GMSB_KCLIQUE_IMPL=warp|lane forces one (A/B measurements, tests); results are identical. */
+ * Kernels for the d+ > 32 sub-problems, chosen from k and the out-degrees: lane-parallel for 5 <= k <= 10,
+ * warp-cooperative otherwise. */
 GMSB_API int gmsb_kclique_count(gmsb_graph_t g, int k, uint64_t *out);
 /* multi-GPU form: this process counts share part_index of part_count of the per-vertex sub-problems (graph
  * replicated, dealt out round-robin in descending size); the shares add up to gmsb_kclique_count's result. */

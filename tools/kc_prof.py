@@ -12,4 +12,4 @@ g.kclique_count(3)
 for _ in range(reps):
     t = time.time()
     c = g.kclique_count(k)
-    print(f"k={k} scale={scale} impl={os.environ.get('GMSB_KCLIQUE_IMPL', 'auto')} count={c} seconds={time.time() - t:.3f}", flush=True)
+    print(f"k={k} scale={scale} count={c} seconds={time.time() - t:.3f}", flush=True)

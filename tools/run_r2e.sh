@@ -2,12 +2,3 @@ set -x
 mkdir -p gpurun_out
 timeout 900 python -m pytest tests -m gpu -x -q > gpurun_out/r2e_pytest.log 2>&1; echo "pytest rc=$?" >> gpurun_out/r2e_pytest.log
 tail -5 gpurun_out/r2e_pytest.log
-GMSB_KCLIQUE_PAIR_MIN=128 timeout 300 python -m pytest tests/test_gpu_clique_lane.py -x -q > gpurun_out/r2e_pytest_pair128.log 2>&1; tail -2 gpurun_out/r2e_pytest_pair128.log
-GMSB_KCLIQUE_HUGE=pair timeout 300 python -m pytest tests/test_gpu_clique_lane.py -x -q > gpurun_out/r2e_pytest_hugepair.log 2>&1; tail -2 gpurun_out/r2e_pytest_hugepair.log
-export GMSB_KCLIQUE_TRACE=1
-GMSB_KCLIQUE_PAIR_MIN=256 timeout 300 python tools/kc_prof.py 20 7 > gpurun_out/r2e_kc_s20_k7_pair256.log 2>&1
-GMSB_KCLIQUE_PAIR_MIN=128 timeout 300 python tools/kc_prof.py 20 7 > gpurun_out/r2e_kc_s20_k7_pair128.log 2>&1
-GMSB_KCLIQUE_HUGE=pair timeout 300 python tools/kc_prof.py 22 6 > gpurun_out/r2e_kc_s22_k6_pair.log 2>&1
-GMSB_KCLIQUE_HUGE=pair GMSB_KCLIQUE_PAIR_MIN=256 timeout 300 python tools/kc_prof.py 22 6 > gpurun_out/r2e_kc_s22_k6_pair256.log 2>&1
-unset GMSB_KCLIQUE_TRACE
-cat gpurun_out/r2e_kc_s20_k7_pair256.log gpurun_out/r2e_kc_s20_k7_pair128.log gpurun_out/r2e_kc_s22_k6_pair.log gpurun_out/r2e_kc_s22_k6_pair256.log
