@@ -510,8 +510,9 @@ void count_warp(const BigVerts &b) {
         ticket.zero();
         DevBuf<uint32_t> spill;
         auto launch = [&](auto kern, int block) {
-            if (smem > 48 * 1024)
-                GMSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            // set on every launch: without it the dynamic part may only take 48 KB minus the static scratch (24.8 KB
+            // for the 1024-thread builds), and a larger value left by an earlier call must not decide what fits
+            GMSB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             int resident = 0;
             GMSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, block, smem));
             GMSB_REQUIRE(resident >= 1, "kclique_count: kernel does not fit on an SM");
