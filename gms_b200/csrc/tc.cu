@@ -759,6 +759,20 @@ void tc_total(Graph &g, const gmsb_tc_options &opt_in, uint64_t *out, gmsb_tc_st
     // the schedule holds this device's share only (the edges into the vertices it owns: ownership does not depend on
     // the order the scatter pass's atomics ran in)
     const int64_t my_items = p.n_items, my_merge = p.n_merge, my_gallop = p.n_gallop;
+    // GMSB_TC_TRACE=1: after every counting launch, one line with the triangles it added (read off the running total,
+    // so each launch is followed by a synchronisation while tracing)
+    const bool trace = std::getenv("GMSB_TC_TRACE") != nullptr;
+    unsigned long long traced = 0;
+    auto trace_class = [&](const char *cls, const char *unit, int64_t cnt, int words) {
+        if (!trace) return;
+        const unsigned long long now = total.get(0);
+        if (words >= 0)
+            std::fprintf(stderr, "[gmsb tc] class=%s %s=%lld words=%d triangles=%llu\n", cls, unit, (long long)cnt,
+                         words, now - traced);
+        else
+            std::fprintf(stderr, "[gmsb tc] class=%s %s=%lld triangles=%llu\n", cls, unit, (long long)cnt, now - traced);
+        traced = now;
+    };
 
     t_bm.start();
     if (my_items) {
@@ -766,7 +780,8 @@ void tc_total(Graph &g, const gmsb_tc_options &opt_in, uint64_t *out, gmsb_tc_st
         DevBuf<unsigned int> tickets(3);
         tickets.zero();
         // one persistent wave per window class (the ticket's free is stream-ordered after the kernels)
-        auto launch = [&](auto kern, int BLOCK, const Item *items, int64_t cnt, int cap_words, unsigned int *ticket) {
+        auto launch = [&](const char *cls, auto kern, int BLOCK, const Item *items, int64_t cnt, int cap_words,
+                          unsigned int *ticket) {
             const int64_t mine = cnt;
             if (mine == 0) return;
             const size_t smem = ((size_t)cap_words + 1) * 4;
@@ -779,12 +794,13 @@ void tc_total(Graph &g, const gmsb_tc_options &opt_in, uint64_t *out, gmsb_tc_st
             kern<<<grid, BLOCK, smem, r.stream>>>(items, mine, (uint32_t)cap_words, d.off.p, d.nbr.p,
                                                   p.desc.p, total.p, ticket);
             launched();
+            trace_class(cls, "items", mine, cap_words);
         };
         const Item *it0 = p.items.p, *it1 = it0 + p.cls_items[0], *it2 = it1 + p.cls_items[1];
         // small windows (<= 55 KB of bitmap): four CTAs of 512 threads per SM = 64 resident warps; wide: three
-        launch(k_tc_bitmap2<512, 4, true>, 512, it0, p.cls_items[0], p.cls_words[0], tickets.p);
-        launch(k_tc_bitmap2<512, 4, false>, 512, it1, p.cls_items[1], p.cls_words[1], tickets.p + 1);
-        launch(k_tc_bitmap2<512, 3, false>, 512, it2, p.cls_items[2], p.cls_words[2], tickets.p + 2);
+        launch("near", k_tc_bitmap2<512, 4, true>, 512, it0, p.cls_items[0], p.cls_words[0], tickets.p);
+        launch("small", k_tc_bitmap2<512, 4, false>, 512, it1, p.cls_items[1], p.cls_words[1], tickets.p + 1);
+        launch("wide", k_tc_bitmap2<512, 3, false>, 512, it2, p.cls_items[2], p.cls_words[2], tickets.p + 2);
     }
     t_bm.stop();
     t_mg.start();
@@ -792,6 +808,7 @@ void tc_total(Graph &g, const gmsb_tc_options &opt_in, uint64_t *out, gmsb_tc_st
         int grid = (int)std::min<int64_t>(ceil_div(my_merge, kMergeWarps), (int64_t)r.sm_count * 16);
         k_tc_merge<<<grid, kMergeWarps * 32, 0, r.stream>>>(p.m_desc.p, p.m_v.p, my_merge, d.off.p, d.nbr.p, total.p);
         launched();
+        trace_class("merge", "edges", my_merge, -1);
     }
     t_mg.stop();
     t_gl.start();
@@ -799,6 +816,7 @@ void tc_total(Graph &g, const gmsb_tc_options &opt_in, uint64_t *out, gmsb_tc_st
         int grid = (int)std::min<int64_t>(ceil_div(my_gallop, 8), (int64_t)r.sm_count * 16);
         k_tc_gallop<<<grid, 256, 0, r.stream>>>(p.g_desc.p, p.g_v.p, my_gallop, d.off.p, d.nbr.p, total.p);
         launched();
+        trace_class("gallop", "edges", my_gallop, -1);
     }
     t_gl.stop();
     *out = total.get(0);
