@@ -468,7 +468,10 @@ inline DevSet &S(gmsb_set_t h) {
     GMSB_REQUIRE(h != nullptr, "null set handle");
     return *reinterpret_cast<DevSet *>(h);
 }
-inline void check_op(int op) { GMSB_REQUIRE(op >= GMSB_SET_INTERSECT && op <= GMSB_SET_DIFFERENCE, "unknown set operation"); }
+inline gmsb_set_op_kind check_op(int op) {
+    GMSB_REQUIRE(op >= GMSB_SET_INTERSECT && op <= GMSB_SET_DIFFERENCE, "unknown set operation");
+    return static_cast<gmsb_set_op_kind>(op);
+}
 }  // namespace
 GMSB_API int gmsb_set_from_host(const int32_t *elems, int64_t count, gmsb_set_t *out) {
     return guarded([&] { GMSB_REQUIRE(out, "null output handle"); rt(); *out = reinterpret_cast<gmsb_set_t>(set_from_host(elems, count)); });
@@ -498,17 +501,17 @@ GMSB_API int gmsb_set_equal(gmsb_set_t a, gmsb_set_t b, int *flag) {
 GMSB_API int gmsb_set_op(int op, gmsb_set_t a, gmsb_set_t b, gmsb_set_t *out) {
     return guarded([&] {
         GMSB_REQUIRE(out, "null output handle");
-        check_op(op);
+        const gmsb_set_op_kind kind = check_op(op);
         DevSet *bs[1] = {&S(b)}, *res[1] = {nullptr};
-        set_op_many(op, S(a), 1, bs, res);
+        set_op_many(kind, S(a), 1, bs, res);
         *out = reinterpret_cast<gmsb_set_t>(res[0]);
     });
 }
 GMSB_API int gmsb_set_op_inplace(int op, gmsb_set_t a, gmsb_set_t b) {
     return guarded([&] {
-        check_op(op);
+        const gmsb_set_op_kind kind = check_op(op);
         DevSet *bs[1] = {&S(b)}, *res[1] = {nullptr};
-        set_op_many(op, S(a), 1, bs, res);
+        set_op_many(kind, S(a), 1, bs, res);
         DevSet &dst = S(a);
         dst.own = std::move(res[0]->own);
         dst.p = dst.own.p;
@@ -519,30 +522,30 @@ GMSB_API int gmsb_set_op_inplace(int op, gmsb_set_t a, gmsb_set_t b) {
 GMSB_API int gmsb_set_op_count(int op, gmsb_set_t a, gmsb_set_t b, uint64_t *out) {
     return guarded([&] {
         GMSB_REQUIRE(out, "null output");
-        check_op(op);
+        const gmsb_set_op_kind kind = check_op(op);
         DevSet *bs[1] = {&S(b)};
-        set_op_count_many(op, S(a), 1, bs, out);
+        set_op_count_many(kind, S(a), 1, bs, out);
     });
 }
 GMSB_API int gmsb_set_op_count_many(int op, gmsb_set_t a, int64_t count, const gmsb_set_t *bs, uint64_t *out) {
     return guarded([&] {
         GMSB_REQUIRE(count >= 0 && (count == 0 || (bs && out)), "set_op_count_many: bad arguments");
-        check_op(op);
-        set_op_count_many(op, S(a), count, reinterpret_cast<DevSet *const *>(bs), out);
+        const gmsb_set_op_kind kind = check_op(op);
+        set_op_count_many(kind, S(a), count, reinterpret_cast<DevSet *const *>(bs), out);
     });
 }
 GMSB_API int gmsb_set_op_many(int op, gmsb_set_t a, int64_t count, const gmsb_set_t *bs, gmsb_set_t *outs) {
     return guarded([&] {
         GMSB_REQUIRE(count >= 0 && (count == 0 || (bs && outs)), "set_op_many: bad arguments");
-        check_op(op);
-        set_op_many(op, S(a), count, reinterpret_cast<DevSet *const *>(bs), reinterpret_cast<DevSet **>(outs));
+        const gmsb_set_op_kind kind = check_op(op);
+        set_op_many(kind, S(a), count, reinterpret_cast<DevSet *const *>(bs), reinterpret_cast<DevSet **>(outs));
     });
 }
 GMSB_API int gmsb_set_op_count_neighbourhoods(int op, gmsb_set_t a, gmsb_graph_t g, gmsb_set_t members, uint64_t *out) {
     return guarded([&] {
-        check_op(op);
+        const gmsb_set_op_kind kind = check_op(op);
         GMSB_REQUIRE(out || S(members).n == 0, "null output");
-        set_op_count_members(op, S(a), G(g), S(members), out);
+        set_op_count_members(kind, S(a), G(g), S(members), out);
     });
 }
 

@@ -9,6 +9,7 @@
 //   warp_merge_count — merge path: the merged sequence is cut into tiles, each tile's slices of A and B are
 //                    staged in shared memory with coalesced loads and every lane walks an equal share of the
 //                    tile's diagonal; O((|A|+|B|)/32) steps per lane, right for balanced pairs.
+// warp_intersect_count picks one of the two by the length ratio (kGallopRatio).
 #pragma once
 #include "common.cuh"
 
@@ -77,6 +78,19 @@ __device__ __forceinline__ uint32_t warp_merge_count(const vid_t *__restrict__ a
         }
     }
     return hits;
+}
+
+// Galloping pays off once the longer list is this many times the shorter one (the set-algebra and ADG pull kernels;
+// the triangle schedule takes its ratio from gmsb_tc_options.gallop_ratio instead).
+constexpr int kGallopRatio = 8;
+
+// |A ∩ B| as a per-lane partial count (caller reduces): galloping for skewed pairs, merge path for balanced ones
+__device__ __forceinline__ uint32_t warp_intersect_count(const vid_t *__restrict__ a, int na, const vid_t *__restrict__ b,
+                                                         int nb, int lane, vid_t *buf) {
+    const int lo = na < nb ? na : nb, hi = na < nb ? nb : na;
+    if (lo == 0) return 0;
+    if ((long long)hi >= (long long)kGallopRatio * lo) return warp_gallop_count(a, na, b, nb, lane);
+    return warp_merge_count(a, na, b, nb, lane, buf);
 }
 
 __device__ __forceinline__ unsigned long long warp_sum(unsigned long long x) {

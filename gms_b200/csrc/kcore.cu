@@ -172,10 +172,7 @@ k_adg_pull(const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, const v
         const eid_t b = off[v];
         const int dv = (int)(off[v + 1] - b);
         if (dv == 0) continue;
-        const int lo = dv < nx ? dv : nx, hi = dv < nx ? nx : dv;
-        unsigned long long c = (long long)hi >= 8ll * lo ? warp_gallop_count(nbr + b, dv, X, nx, lane)
-                                                         : warp_merge_count(nbr + b, dv, X, nx, lane, stage[wib]);
-        c = warp_sum(c);
+        const unsigned long long c = warp_sum(warp_intersect_count(nbr + b, dv, X, nx, lane, stage[wib]));
         if (lane == 0 && c) deg[v] -= (int)c;
     }
 }

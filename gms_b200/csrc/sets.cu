@@ -3,128 +3,21 @@
 // Replaces (as a drop-in type for algorithms written against the Set concept, SURVEY.md 8b):
 //   SortedSetBase<int32_t>            gms/representations/sets/sorted_set.h:22-270
 //   SortedSetRefBase<int32_t>         gms/representations/sets/sorted_set_ref.h:10-80   (borrowed neighbourhoods)
-//   vec_set_{union,intersect,intersect_count,difference}   sets/sorted_set_operations.h:30-106
 //
 // A set is an ascending, duplicate-free int32 array in HBM — owned, or borrowed from a graph's CSR like SortedSetRef.
-// Every binary operation takes SET HANDLES and leaves its result on the device, so a chain such as the
-// Bron-Kerbosch step  P' = P ∩ N(v), X' = X ∩ N(v), P = P \ {v}  (maximal_clique_enum/sequential/tomita.h:17-60) or the
-// pull step of the approximate degeneracy order (preprocessing/parallel/degeneracy_approx_set.h:60-80) never
-// returns to the host.  The "many" forms run one left set against a batch of right sets (or against the
-// neighbourhoods of the members of a set) in one launch: one warp per pair, the same kernels as the batched
-// neighbourhood API in setops.cu (galloping for skewed pairs, merge path for balanced ones).
+// This file holds the object: construct (sorting what it is given), range, neighbourhood view, clone, find, add /
+// remove, equality, copy to the host.  Its binary operations (vec_set_{union,intersect,intersect_count,difference},
+// sets/sorted_set_operations.h:30-106) take SET HANDLES and leave their result on the device, so a chain such as the
+// Bron-Kerbosch step  P' = P ∩ N(v), X' = X ∩ N(v), P = P \ {v}  (maximal_clique_enum/sequential/tomita.h:17-60) never
+// returns to the host; they run on the same kernels as the batched neighbourhood API, in setops.cu.
 #include "common.cuh"
 #include "sort.cuh"
 #include "isect.cuh"
-#include "ops.cuh"
 #include "sets.cuh"
-
-#include <vector>
 
 namespace gmsb {
 
 namespace {
-
-constexpr int kWarps = 8;
-constexpr int kGallopRatio = 8;
-
-struct Span {
-    const vid_t *p;
-    int64_t n;
-};
-
-__device__ __forceinline__ uint32_t span_count(const vid_t *a, int na, const vid_t *b, int nb, int lane, vid_t *buf) {
-    const int lo = na < nb ? na : nb, hi = na < nb ? nb : na;
-    if (lo == 0) return 0;
-    if ((long long)hi >= (long long)kGallopRatio * lo) return warp_gallop_count(a, na, b, nb, lane);
-    return warp_merge_count(a, na, b, nb, lane, buf);
-}
-
-// out[i] = |A ∩ B_i| (op 0) or |A ∪ B_i| (op 1) or |A \ B_i| (op 2); `left` is one span shared by all pairs
-__global__ void __launch_bounds__(kWarps * 32)
-k_span_count(Span left, const Span *__restrict__ right, int64_t np, int op, unsigned long long *__restrict__ out) {
-    __shared__ vid_t stage[kWarps][kMergeTile + 2];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
-    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    for (int64_t i = warp; i < np; i += nwarps) {
-        const Span b = right[i];
-        unsigned long long c = span_count(left.p, (int)left.n, b.p, (int)b.n, lane, stage[wib]);
-        c = warp_sum(c);
-        if (lane == 0)
-            out[i] = op == 0 ? c : (op == 1 ? (unsigned long long)left.n + (unsigned long long)b.n - c
-                                            : (unsigned long long)left.n - c);
-    }
-}
-// neighbourhoods of the listed vertices as the right-hand spans
-__global__ void k_neighbourhood_spans(const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, int64_t n,
-                                      const vid_t *__restrict__ verts, int64_t nv, Span *__restrict__ out,
-                                      int *__restrict__ bad) {
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < nv; i += (int64_t)gridDim.x * blockDim.x) {
-        const vid_t v = verts[i];
-        if (v < 0 || v >= n) { *bad = 1; out[i] = Span{nullptr, 0}; continue; }
-        out[i] = Span{nbr + off[v], off[v + 1] - off[v]};
-    }
-}
-
-// Materialising A op B_i, ascending, two passes (count, then write at out_off[i]); one warp per pair.
-//   op 0 intersect: elements of the shorter list found in the longer one      (std::set_intersection)
-//   op 2 difference: elements of A not found in B                              (std::set_difference)
-//   op 1 union: every element computes its own slot — j + lower_bound(other, x) - common elements before it
-template <int OP>
-__global__ void __launch_bounds__(256)
-k_span_op(Span left, const Span *__restrict__ right, int64_t np, int64_t *__restrict__ counts,
-          const int64_t *__restrict__ out_off, vid_t *__restrict__ out_elems) {
-    const int lane = threadIdx.x & 31;
-    const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
-    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    for (int64_t i = warp; i < np; i += nwarps) {
-        const vid_t *a = left.p, *b = right[i].p;
-        int na = (int)left.n, nb = (int)right[i].n;
-        if (OP == 0 && na > nb) { const vid_t *t = a; a = b; b = t; const int tn = na; na = nb; nb = tn; }
-        const int64_t w = out_elems ? out_off[i] : 0;
-        int64_t c = 0;
-        int common = 0;
-        for (int j0 = 0; j0 < na; j0 += 32) {
-            const int j = j0 + lane;
-            bool hit = false;
-            int lo = 0;
-            vid_t x = 0;
-            if (j < na) {
-                x = a[j];
-                lo = lower_bound_dev(b, nb, x);
-                hit = lo < nb && b[lo] == x;
-            }
-            const bool keep = OP == 0 ? hit : (OP == 2 ? (j < na && !hit) : j < na);
-            const unsigned hmask = __ballot_sync(0xffffffffu, hit), kmask = __ballot_sync(0xffffffffu, keep);
-            if (out_elems && keep) {
-                if (OP == 1) out_elems[w + j + lo - (common + __popc(hmask & ((1u << lane) - 1)))] = x;
-                else out_elems[w + c + __popc(kmask & ((1u << lane) - 1))] = x;
-            }
-            c += __popc(kmask);
-            common += __popc(hmask);
-        }
-        if (OP == 1) {
-            if (!out_elems) { if (lane == 0) counts[i] = (int64_t)na + nb - common; continue; }
-            common = 0;
-            for (int t0 = 0; t0 < nb; t0 += 32) {
-                const int t = t0 + lane;
-                bool hit = false;
-                int lo = 0;
-                vid_t x = 0;
-                if (t < nb) {
-                    x = b[t];
-                    lo = lower_bound_dev(a, na, x);
-                    hit = lo < na && a[lo] == x;
-                }
-                const unsigned hmask = __ballot_sync(0xffffffffu, hit);
-                if (t < nb && !hit) out_elems[w + t + lo - (common + __popc(hmask & ((1u << lane) - 1)))] = x;
-                common += __popc(hmask);
-            }
-        } else if (!out_elems && lane == 0) {
-            counts[i] = c;
-        }
-    }
-}
 
 __global__ void k_iota(vid_t *__restrict__ out, int64_t n) {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
@@ -148,16 +41,6 @@ __global__ void k_insert(const vid_t *__restrict__ in, int64_t n, int64_t pos, v
 __global__ void k_erase(const vid_t *__restrict__ in, int64_t n, int64_t pos, vid_t *__restrict__ out) {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i + 1 < n; i += (int64_t)gridDim.x * blockDim.x)
         out[i] = i < pos ? in[i] : in[i + 1];
-}
-
-Span span_of(const DevSet &s) { return Span{s.p, s.n}; }
-
-template <typename K>
-void launch_op(int op, K k0, K k1, K k2, int grid, Span left, const Span *right, int64_t np, int64_t *counts,
-               const int64_t *out_off, vid_t *out_elems) {
-    Runtime &r = rt();
-    (op == 0 ? k0 : (op == 1 ? k1 : k2))<<<grid, 256, 0, r.stream>>>(left, right, np, counts, out_off, out_elems);
-    launched();
 }
 
 }  // namespace
@@ -282,66 +165,6 @@ void set_remove(DevSet &a, vid_t x) {
     a.own = std::move(shrunk);
     a.p = a.own.p;
     a.n -= 1;
-}
-
-// counts[i] for one left set against np right spans (device array)
-static void count_spans(const DevSet &a, const Span *right_dev, int64_t np, int op, uint64_t *out_host) {
-    Runtime &r = rt();
-    DevBuf<unsigned long long> out((size_t)np);
-    const int grid = (int)std::min<int64_t>(ceil_div(np, kWarps), (int64_t)r.sm_count * 16);
-    k_span_count<<<grid, kWarps * 32, 0, r.stream>>>(span_of(a), right_dev, np, op, out.p); launched();
-    out.download(reinterpret_cast<unsigned long long *>(out_host), (size_t)np);
-}
-
-void set_op_count_many(int op, const DevSet &a, int64_t np, DevSet *const *bs, uint64_t *out) {
-    GMSB_REQUIRE(op >= 0 && op <= 2, "set op: unknown operation");
-    if (np == 0) return;
-    std::vector<Span> h((size_t)np);
-    for (int64_t i = 0; i < np; ++i) { GMSB_REQUIRE(bs[i] != nullptr, "set op: null set handle"); h[i] = span_of(*bs[i]); }
-    DevBuf<Span> d((size_t)np);
-    d.upload(h.data(), (size_t)np);
-    count_spans(a, d.p, np, op, out);
-}
-
-void set_op_count_members(int op, const DevSet &a, Graph &g, const DevSet &members, uint64_t *out) {
-    GMSB_REQUIRE(op >= 0 && op <= 2, "set op: unknown operation");
-    if (members.n == 0) return;
-    Runtime &r = rt();
-    DevBuf<Span> d((size_t)members.n);
-    DevBuf<int> bad(1);
-    bad.zero();
-    k_neighbourhood_spans<<<grid_for(members.n, 256), 256, 0, r.stream>>>(g.off.p, g.nbr.p, g.n, members.p, members.n,
-                                                                        d.p, bad.p);
-    launched();
-    GMSB_REQUIRE(bad.get(0) == 0, "set op: member outside the graph");
-    count_spans(a, d.p, members.n, op, out);
-}
-
-void set_op_many(int op, const DevSet &a, int64_t np, DevSet *const *bs, DevSet **outs) {
-    GMSB_REQUIRE(op >= 0 && op <= 2, "set op: unknown operation");
-    if (np == 0) return;
-    Runtime &r = rt();
-    std::vector<Span> h((size_t)np);
-    for (int64_t i = 0; i < np; ++i) { GMSB_REQUIRE(bs[i] != nullptr, "set op: null set handle"); h[i] = span_of(*bs[i]); }
-    DevBuf<Span> d((size_t)np);
-    d.upload(h.data(), (size_t)np);
-    DevBuf<int64_t> counts((size_t)np + 1), offs((size_t)np + 1);
-    counts.zero();
-    const int grid = (int)std::min<int64_t>(ceil_div(np, 8), (int64_t)r.sm_count * 16);
-    launch_op(op, k_span_op<0>, k_span_op<1>, k_span_op<2>, grid, span_of(a), d.p, np, counts.p, nullptr, nullptr);
-    exclusive_sum(counts.p, offs.p, np + 1);
-    std::vector<int64_t> ho((size_t)np + 1);
-    offs.download(ho.data(), (size_t)np + 1);
-    DevBuf<vid_t> elems((size_t)ho[np]);
-    if (ho[np])
-        launch_op(op, k_span_op<0>, k_span_op<1>, k_span_op<2>, grid, span_of(a), d.p, np, nullptr, offs.p, elems.p);
-    std::vector<DevSet *> made;
-    try {
-        for (int64_t i = 0; i < np; ++i) {
-            made.push_back(set_from_device(elems.p + ho[i], ho[i + 1] - ho[i], true));
-            outs[i] = made.back();
-        }
-    } catch (...) { for (auto *m : made) delete m; throw; }
 }
 
 }  // namespace gmsb

@@ -1,4 +1,5 @@
-// sets.cuh — device-resident sorted set (sets.cu) behind the gmsb_set_* entry points.
+// sets.cuh — device-resident sorted set (sets.cu) behind the gmsb_set_* entry points; its binary operations are in
+// setops.cu.
 #pragma once
 #include "common.cuh"
 
@@ -8,6 +9,12 @@ struct DevSet {
     DevBuf<vid_t> own;          // storage of an owning set; empty for a view borrowed from a graph's CSR
     const vid_t *p = nullptr;   // ascending, duplicate-free
     int64_t n = 0;
+};
+
+// an ascending list in device memory: a set's elements or a neighbourhood
+struct Span {
+    const vid_t *p;
+    int64_t n;
 };
 
 DevSet *set_from_host(const vid_t *elems, int64_t count);
@@ -20,9 +27,9 @@ bool set_contains(const DevSet &a, vid_t x);
 bool set_equal(const DevSet &a, const DevSet &b);
 void set_add(DevSet &a, vid_t x);
 void set_remove(DevSet &a, vid_t x);
-// op: 0 intersect, 1 union, 2 difference (left minus right)
-void set_op_count_many(int op, const DevSet &a, int64_t np, DevSet *const *bs, uint64_t *out);
-void set_op_count_members(int op, const DevSet &a, Graph &g, const DevSet &members, uint64_t *out);
-void set_op_many(int op, const DevSet &a, int64_t np, DevSet *const *bs, DevSet **outs);
+// setops.cu; difference is left minus right
+void set_op_count_many(gmsb_set_op_kind op, const DevSet &a, int64_t np, DevSet *const *bs, uint64_t *out);
+void set_op_count_members(gmsb_set_op_kind op, const DevSet &a, Graph &g, const DevSet &members, uint64_t *out);
+void set_op_many(gmsb_set_op_kind op, const DevSet &a, int64_t np, DevSet *const *bs, DevSet **outs);
 
 }  // namespace gmsb

@@ -265,8 +265,28 @@ def test_pair_ops_against_oracle(gms, orc, seed):
     finite = np.isfinite(ref_)
     assert (np.isfinite(got) == finite).all()
     assert np.allclose(got[finite], ref_[finite], rtol=1e-13, atol=0)
-    with pytest.raises(gms.GmsbError):
-        g.intersect_count_batch(np.array([0, g.n], np.int32), np.array([0, 0], np.int32))
+    for call in (g.intersect_count_batch, g.union_count_batch, g.intersect_batch, g.difference_batch, g.union_batch):
+        for x, y in (([0, g.n], [0, 0]), ([0, 0], [-1, 0])):
+            with pytest.raises(gms.GmsbError, match="vertex id out of range"):
+                call(np.array(x, np.int32), np.array(y, np.int32))
+    # out-lists of 64, 511 and 512 elements: pairs on both sides of the count kernels' gallop rule (longer >= 8 x
+    # shorter), in both orders, through the batch API
+    src, dst = [], []
+    for v, deg in ((0, 64), (1, 511), (2, 512)):
+        src += [v] * deg
+        dst += rng.choice(np.arange(3, 1200), deg, replace=False).tolist()
+    gb, ob = gms.Graph.from_edgelist(src, dst, False), orc.from_el(src, dst, False)
+    boff, bnbr = ob.csr()
+    lists = [bnbr[boff[v]:boff[v + 1]] for v in range(3)]
+    assert [len(x) for x in lists] == [64, 511, 512]
+    pa, pb = np.array([0, 0, 2, 1], np.int32), np.array([2, 1, 0, 0], np.int32)
+    assert gb.intersect_count_batch(pa, pb).tolist() == [orc.intersect_count(lists[x], lists[y]) for x, y in zip(pa, pb)]
+    assert gb.union_count_batch(pa, pb).tolist() == [orc.union_count(lists[x], lists[y]) for x, y in zip(pa, pb)]
+    for batch, op in ((gb.intersect_batch, orc.intersect), (gb.difference_batch, orc.difference),
+                      (gb.union_batch, orc.union)):
+        boffs, belems = batch(pa, pb)
+        for i, (x, y) in enumerate(zip(pa, pb)):
+            assert belems[boffs[i]:boffs[i + 1]].tolist() == op(lists[x], lists[y]).tolist()
 
 
 def test_orientation_fallback_path(gms, orc, monkeypatch):

@@ -10,18 +10,24 @@ pytestmark = pytest.mark.gpu
 
 
 def rand_set(rng, n, hi):
-    return np.unique(rng.integers(0, hi, n)).astype(np.int32)
+    return np.sort(rng.choice(hi, n, replace=False)).astype(np.int32)       # exactly n elements
 
 
 def test_binary_operations_against_the_oracle(gms, orc):
     rng = np.random.default_rng(11)
-    sizes = [(0, 0), (0, 50), (1, 1), (5, 4000), (4000, 5), (700, 900), (3000, 3000), (33, 32), (20000, 150)]
+    # (64, 512) / (512, 64) sit on the gallop side of the count kernels' rule (longer >= 8 x shorter), (64, 511) /
+    # (511, 64) one element below it, on the merge side
+    sizes = [(0, 0), (0, 50), (1, 1), (5, 4000), (4000, 5), (700, 900), (3000, 3000), (33, 32), (20000, 150),
+             (64, 512), (64, 511), (512, 64), (511, 64)]
     for na, nb in sizes:
         a, b = rand_set(rng, na, 50000), rand_set(rng, nb, 50000)
         A, B = gms.DeviceSet(rng.permutation(a)), gms.DeviceSet(b)        # the constructor sorts
         assert (A.to_array() == a).all()
         assert A.op_count("intersect", B) == orc.intersect_count(a, b)
         assert A.op_count("union", B) == orc.union_count(a, b)
+        assert A.op_count("difference", B) == len(orc.difference(a, b))
+        assert B.op_count("difference", A) == len(orc.difference(b, a))
+        assert list(A.op_count_many("intersect", [B, A])) == [orc.intersect_count(a, b), na]
         assert (A.op("intersect", B).to_array() == orc.intersect(a, b)).all()
         assert (A.op("union", B).to_array() == orc.union(a, b)).all()
         assert (A.op("difference", B).to_array() == orc.difference(a, b)).all()
@@ -56,14 +62,15 @@ def test_one_set_against_many_and_against_neighbourhoods(gms, orc):
     p = rand_set(rng, 200, g.n)
     P = gms.DeviceSet(p)
     members = gms.DeviceSet(rand_set(rng, 120, g.n))
-    got = P.op_count_neighbourhoods("intersect", g, members)
-    want = [orc.intersect_count(p, nbr[off[v]:off[v + 1]]) for v in members.to_array()]
-    assert list(got) == want
     views = [gms.DeviceSet.neighbourhood(g, int(v)) for v in members.to_array()[:40]]
-    assert list(P.op_count_many("intersect", views)) == want[:40]
-    outs = P.op_many("intersect", views)
-    for v, r in zip(members.to_array()[:40], outs):
-        assert (r.to_array() == orc.intersect(p, nbr[off[v]:off[v + 1]])).all()
+    difference_count = lambda x, y: len(orc.difference(x, y))                # noqa: E731
+    for kind, op, count in (("intersect", orc.intersect, orc.intersect_count), ("union", orc.union, orc.union_count),
+                            ("difference", orc.difference, difference_count)):
+        want = [count(p, nbr[off[v]:off[v + 1]]) for v in members.to_array()]
+        assert list(P.op_count_neighbourhoods(kind, g, members)) == want, kind
+        assert list(P.op_count_many(kind, views)) == want[:40], kind
+        for v, r in zip(members.to_array()[:40], P.op_many(kind, views)):
+            assert (r.to_array() == op(p, nbr[off[v]:off[v + 1]])).all(), kind
     # a view turns into an owning set when it is modified; the graph is untouched
     view = gms.DeviceSet.neighbourhood(g, 7)
     before = view.to_array().copy()

@@ -6,8 +6,8 @@ One JSON line per measurement:
   * edge_similarity (Jaccard, CommNeigh: from one pass of the oriented triangle schedule; Adamic-Adar: one symmetric-list
     intersection per edge, the batched intersect kernels) over ALL undirected edges, with the bytes that bound each:
     B_TC for the support path, B_sim = sum over edges u<v of 4 (d(u) + d(v)) + 8 m for the pair path (SURVEY.md 8d);
-  * gmsb_intersect_count_batch / gmsb_pair_similarity on hub x hub pairs (both lists long and balanced: the block-compare
-    kernel) and on hub x leaf pairs (skewed: the galloping kernel), host arrays in, host arrays out;
+  * gmsb_intersect_count_batch / gmsb_pair_similarity on hub x hub pairs (both lists long and balanced: the merge
+    path) and on hub x leaf pairs (skewed: galloping), host arrays in, host arrays out;
   * the reference's CPU loop over vertex_similarity<Jaccard|CommNeigh> on a bounded sample of the same edges."""
 import argparse
 import json
