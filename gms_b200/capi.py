@@ -83,6 +83,8 @@ SIGNATURES = {
     "gmsb_graph_free": (C.c_int, [C.c_void_p]),
     "gmsb_order_degree": (C.c_int, [C.c_void_p, C.c_int, _i32p]),
     "gmsb_order_degeneracy": (C.c_int, [C.c_void_p, _i32p]),
+    "gmsb_core_numbers": (C.c_int, [C.c_void_p, _i32p]),
+    "gmsb_truss_numbers": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_int64)]),
     "gmsb_order_degeneracy_approx": (C.c_int, [C.c_void_p, C.c_double, C.c_int, _i32p]),
     "gmsb_order_degeneracy_approx_ex": (C.c_int, [C.c_void_p, C.c_double, C.c_int, C.c_int, C.c_int, C.c_uint64, _i32p]),
     "gmsb_graph_worth_relabelling": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
@@ -303,6 +305,20 @@ class Graph:
         out = np.zeros(max(self.n, 1), np.int32)
         _check(lib().gmsb_order_degeneracy(self.h, out))
         return out[:self.n]
+
+    def core_numbers(self):
+        """Core number of every vertex (int32[n]); the maximum is the degeneracy."""
+        out = np.zeros(max(self.n, 1), np.int32)
+        _check(lib().gmsb_core_numbers(self.h, out))
+        return out[:self.n]
+
+    def truss_numbers(self):
+        """Truss number of every undirected edge u<v (int32[m]), in the edge order of edge_similarity."""
+        m = C.c_int64(0)
+        _check(lib().gmsb_truss_numbers(self.h, None, C.byref(m)))
+        out = np.zeros(max(m.value, 1), np.int32)
+        _check(lib().gmsb_truss_numbers(self.h, out.ctypes.data, C.byref(m)))
+        return out[:m.value]
 
     def degeneracy_order_approx(self, epsilon=1.0, rank_format=False):
         out = np.zeros(max(self.n, 1), np.int32)

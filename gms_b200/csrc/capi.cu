@@ -345,6 +345,16 @@ GMSB_API int gmsb_order_degeneracy(gmsb_graph_t g, int32_t *out_rank) {
         degeneracy_rank(gr, out_rank);
     });
 }
+GMSB_API int gmsb_core_numbers(gmsb_graph_t g, int32_t *out_n) {
+    return guarded([&] {
+        Graph &gr = G(g);
+        GMSB_REQUIRE(out_n || gr.n == 0, "null output");
+        core_numbers(gr, out_n);
+    });
+}
+GMSB_API int gmsb_truss_numbers(gmsb_graph_t g, int32_t *out, int64_t *m_out) {
+    return guarded([&] { truss_numbers(G(g), out, m_out); });
+}
 GMSB_API int gmsb_order_degeneracy_approx(gmsb_graph_t g, double epsilon, int rank_format, int32_t *out) {
     return guarded([&] {
         Graph &gr = G(g);

@@ -1,4 +1,4 @@
-// kcore.cu — degeneracy ordering by parallel k-core peeling.
+// kcore.cu — degeneracy ordering and core numbers by parallel k-core peeling.
 //
 // Replaces  PpSequential::getDegeneracyOrderingDanischHeap   gms/algorithms/preprocessing/sequential/degeneracy_danisch.h:12-56
 //
@@ -35,10 +35,13 @@ __global__ void k_collect(int64_t n, int k, const int *__restrict__ deg, int *__
         }
 }
 
-__global__ void k_assign_rank(const vid_t *__restrict__ queue, int qs, int64_t n, int64_t done,
-                              vid_t *__restrict__ rank) {
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < qs; i += gridDim.x * blockDim.x)
-        rank[queue[i]] = (vid_t)(n - 1 - (done + i));
+// removal rank (when rank != nullptr) and core number (when core != nullptr) of the frontier's vertices
+__global__ void k_assign_level(const vid_t *__restrict__ queue, int qs, int64_t n, int64_t done, int k,
+                               vid_t *__restrict__ rank, int32_t *__restrict__ core) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < qs; i += gridDim.x * blockDim.x) {
+        if (rank) rank[queue[i]] = (vid_t)(n - 1 - (done + i));
+        if (core) core[queue[i]] = k;
+    }
 }
 
 // one warp per frontier vertex: decrement live neighbours; those that reach <= k join the next frontier
@@ -61,14 +64,14 @@ __global__ void k_relax(const eid_t *__restrict__ off, const vid_t *__restrict__
 
 }  // namespace
 
-void degeneracy_rank(Graph &g, vid_t *out_rank) {
-    GMSB_REQUIRE(!g.directed, "order_degeneracy: graph must be undirected");
+// The level-by-level peel.  A vertex that leaves at level k has core number k: after level k-1 has drained, every
+// remaining vertex has residual degree >= k, so the remaining graph is the k-core.  Writes the removal rank and/or
+// the core number of every vertex (device arrays; either may be null).
+static void peel_levels(Graph &g, vid_t *rank, int32_t *core) {
     Runtime &r = rt();
     const int64_t n = g.n;
-    if (n == 0) return;
-    GMSB_REQUIRE(n < (int64_t(1) << 31), "order_degeneracy: too many vertices");
     DevBuf<int> deg(n), gone(n), sizes(2);
-    DevBuf<vid_t> qa(n), qb(n), rank(n);
+    DevBuf<vid_t> qa(n), qb(n);
     gone.zero();
     k_init_degrees<<<grid_for(n, 256), 256, 0, r.stream>>>(g.off.p, n, deg.p); launched();
     int64_t done = 0;
@@ -82,7 +85,7 @@ void degeneracy_rank(Graph &g, vid_t *out_rank) {
             GMSB_CUDA(cudaMemcpyAsync(&qs, cs, sizeof(int), cudaMemcpyDeviceToHost, r.stream));
             GMSB_CUDA(cudaStreamSynchronize(r.stream));
             if (qs == 0) break;
-            k_assign_rank<<<grid_for(qs, 256), 256, 0, r.stream>>>(cur, qs, n, done, rank.p); launched();
+            k_assign_level<<<grid_for(qs, 256), 256, 0, r.stream>>>(cur, qs, n, done, k, rank, core); launched();
             done += qs;
             GMSB_CUDA(cudaMemsetAsync(ns, 0, sizeof(int), r.stream));
             k_relax<<<grid_for((int64_t)qs * 32, 256), 256, 0, r.stream>>>(g.off.p, g.nbr.p, cur, qs, k, deg.p, gone.p,
@@ -92,7 +95,26 @@ void degeneracy_rank(Graph &g, vid_t *out_rank) {
             std::swap(cs, ns);
         }
     }
+}
+
+void degeneracy_rank(Graph &g, vid_t *out_rank) {
+    GMSB_REQUIRE(!g.directed, "order_degeneracy: graph must be undirected");
+    const int64_t n = g.n;
+    if (n == 0) return;
+    GMSB_REQUIRE(n < (int64_t(1) << 31), "order_degeneracy: too many vertices");
+    DevBuf<vid_t> rank(n);
+    peel_levels(g, rank.p, nullptr);
     rank.download(out_rank, n);
+}
+
+void core_numbers(Graph &g, int32_t *out_core) {
+    GMSB_REQUIRE(!g.directed, "core_numbers: graph must be undirected");
+    const int64_t n = g.n;
+    if (n == 0) return;
+    GMSB_REQUIRE(n < (int64_t(1) << 31), "core_numbers: too many vertices");
+    DevBuf<int32_t> core(n);
+    peel_levels(g, nullptr, core.p);
+    core.download(out_core, n);
 }
 
 // ---- approximate degeneracy order (ADG) ---------------------------------------------------------------------------------

@@ -28,6 +28,7 @@ void support_to_vertex2(Graph &g, const uint32_t *sup, unsigned long long *t2_de
 void vertex2_unrank(Graph &g, const unsigned long long *t2_dev, int64_t *out_dev);
 void edge_scores_range(Graph &g, int metric, const int64_t *base_dev, const uint32_t *sup, int64_t a_begin, int64_t a_end,
                        double *out_dev);
+void edge_support(Graph &g, const int64_t *base_dev, uint32_t *out_dev);
 void upper_edge_base(Graph &g, DevBuf<int64_t> &base, int64_t *m_out);      // setops.cu: scan of per-vertex counts of neighbours > vertex
 void emit_upper_pairs(Graph &g, const int64_t *base_dev, vid_t *pa, vid_t *pb);
 void pair_similarity_device(Graph &g, int metric, int64_t np, const vid_t *da, const vid_t *db, double *out_host);
@@ -43,6 +44,10 @@ void mg_release(Graph &g);
 
 // kcore.cu
 void degeneracy_rank(Graph &g, vid_t *out_rank);
+void core_numbers(Graph &g, int32_t *out_core);
+
+// truss.cu
+void truss_numbers(Graph &g, int32_t *out, int64_t *m_out);
 void degeneracy_order_approx(Graph &g, double epsilon, bool rank_format, vid_t *out_host);
 void degeneracy_order_approx_ex(Graph &g, double epsilon, bool rank_format, int boundary, bool pull, uint64_t seed,
                                 vid_t *out_host);

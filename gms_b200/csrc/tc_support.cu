@@ -165,6 +165,14 @@ __global__ void k_unrank(const unsigned long long *__restrict__ t2, const vid_t 
         out[order[r]] = (int64_t)t2[r];
 }
 
+// support of the undirected edge between rank-space vertices ra and rb, read from its oriented copy
+__device__ __forceinline__ uint32_t oriented_support(vid_t ra, vid_t rb, const eid_t *__restrict__ doff,
+                                                     const vid_t *__restrict__ dnbr, const uint32_t *__restrict__ sup) {
+    const vid_t lo = ra < rb ? ra : rb, hi = ra < rb ? rb : ra;
+    const eid_t lb = doff[lo];
+    return sup[lb + lower_bound_dev(dnbr + lb, (int)(doff[lo + 1] - lb), hi)];
+}
+
 // Score of every undirected edge a<b (CSR order of the ORIGINAL graph) from the support of its oriented copy.
 __global__ void k_edge_scores(const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, int64_t a_begin, int64_t n,
                               const int64_t *__restrict__ base, const vid_t *__restrict__ rank,
@@ -181,12 +189,8 @@ __global__ void k_edge_scores(const eid_t *__restrict__ off, const vid_t *__rest
         const vid_t ra = rank[a];
         for (int64_t j = lane; j < c; j += 32) {
             const vid_t b = nbr[s0 + j];
-            const vid_t rb = rank[b];
             const unsigned long long db = (unsigned long long)(off[b + 1] - off[b]);
-            const vid_t lo = ra < rb ? ra : rb, hi = ra < rb ? rb : ra;
-            const eid_t lb = doff[lo];
-            const int pos = lower_bound_dev(dnbr + lb, (int)(doff[lo + 1] - lb), hi);
-            const unsigned long long cnt = sup[lb + pos];
+            const unsigned long long cnt = oriented_support(ra, rank[b], doff, dnbr, sup);
             const double cd = (double)cnt;
             double score;
             if (metric == GMSB_SIM_JACCARD) score = (da == 0 && db == 0) ? 1.0 : cd / (double)(da + db + cd);
@@ -196,6 +200,22 @@ __global__ void k_edge_scores(const eid_t *__restrict__ off, const vid_t *__rest
             else score = (double)(da * db);
             out[base[a] + j] = score;
         }
+    }
+}
+
+// Support of every undirected edge a<b, indexed like k_edge_scores' output (the edge ids of truss.cu).
+__global__ void k_edge_support(const eid_t *__restrict__ off, const vid_t *__restrict__ nbr, int64_t n,
+                               const int64_t *__restrict__ base, const vid_t *__restrict__ rank,
+                               const eid_t *__restrict__ doff, const vid_t *__restrict__ dnbr,
+                               const uint32_t *__restrict__ sup, uint32_t *__restrict__ out) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t a = warp; a < n; a += nwarps) {
+        const int64_t c = base[a + 1] - base[a];
+        const eid_t s0 = off[a + 1] - c;
+        const vid_t ra = rank[a];
+        for (int64_t j = lane; j < c; j += 32) out[base[a] + j] = oriented_support(ra, rank[nbr[s0 + j]], doff, dnbr, sup);
     }
 }
 
@@ -283,6 +303,17 @@ void edge_scores_range(Graph &g, int metric, const int64_t *base_dev, const uint
     k_edge_scores<<<grid_for((a_end - a_begin) * 32, 256), 256, 0, r.stream>>>(g.off.p, g.nbr.p, a_begin, a_end, base_dev,
                                                                              d.rank.p, d.off.p, d.nbr.p, sup, metric,
                                                                              out_dev);
+    launched();
+}
+
+// triangle support of every undirected edge a<b in edge-id order (out_dev: uint32[m]); `base` as below
+void edge_support(Graph &g, const int64_t *base_dev, uint32_t *out_dev) {
+    Runtime &r = rt();
+    DevBuf<uint32_t> sup;
+    tc_support(g, sup);
+    Dag &d = *g.dag;
+    k_edge_support<<<grid_for(g.n * 32, 256), 256, 0, r.stream>>>(g.off.p, g.nbr.p, g.n, base_dev, d.rank.p, d.off.p,
+                                                                d.nbr.p, sup.p, out_dev);
     launched();
 }
 

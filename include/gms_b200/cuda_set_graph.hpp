@@ -276,6 +276,20 @@ inline void degeneracy_ordering(const CudaSetGraph &g, Output &ranking) {
     check(gmsb_order_degeneracy(g.handle(), tmp.data()));
     for (int64_t i = 0; i < n; ++i) ranking[i] = tmp[i];
 }
+// core number of every vertex (the largest k whose k-core holds it); the maximum is the degeneracy
+inline std::vector<int32_t> core_numbers(const CudaSetGraph &g) {
+    std::vector<int32_t> out(static_cast<size_t>(g.num_nodes()));
+    check(gmsb_core_numbers(g.handle(), out.data()));
+    return out;
+}
+// truss number of every undirected edge u<v, in the edge order of edge_similarity
+inline std::vector<int32_t> truss_numbers(const CudaSetGraph &g) {
+    int64_t cnt = 0;
+    check(gmsb_truss_numbers(g.handle(), nullptr, &cnt));
+    std::vector<int32_t> out(static_cast<size_t>(cnt));
+    if (cnt) check(gmsb_truss_numbers(g.handle(), out.data(), &cnt));
+    return out;
+}
 // approximate degeneracy order, averageDegree boundary (degeneracy_approx_csr.h:13-78); ascending convention
 template <bool useRankFormat = false, class Output = std::vector<NodeId>>
 inline void degeneracy_ordering_approx(const CudaSetGraph &g, Output &res, double epsilon) {

@@ -142,6 +142,16 @@ GMSB_API int gmsb_order_degeneracy(gmsb_graph_t g, int32_t *out_rank);
  * rounds remove every vertex with residual degree <= (1+eps)*average; inside a round vertices are ordered by that
  * degree (ties by id; unspecified in the reference). Ascending convention: first removed = position / rank 0. */
 GMSB_API int gmsb_order_degeneracy_approx(gmsb_graph_t g, double epsilon, int rank_format, int32_t *out);
+/* Core number of every vertex: the largest k such that v belongs to the k-core (the maximal subgraph of minimum
+ * degree >= k); 0 for an isolated vertex; max over v = the degeneracy.  Undirected graphs only.  GMS has no per-vertex
+ * core numbers (its verifiers report the maximum of an order); the value is what the peel of gmsb_order_degeneracy
+ * reaches when it removes the vertex. */
+GMSB_API int gmsb_core_numbers(gmsb_graph_t g, int32_t *out_n);
+/* Truss number of every undirected edge a<b, in the CSR order of gmsb_edge_similarity: the largest k such that the
+ * edge belongs to the k-truss (the maximal subgraph in which every edge lies in >= k-2 triangles of the subgraph);
+ * 2 for an edge in no triangle.  Two-pass like gmsb_edge_similarity: out may be NULL, *m_out = number of edges.
+ * Undirected graphs with fewer than 2^31 edges only (GMSB_ERR_INVALID otherwise). */
+GMSB_API int gmsb_truss_numbers(gmsb_graph_t g, int32_t *out, int64_t *m_out);
 /* getDegeneracyOrderingApprox{CGraph,SGraph}<boundary, useRankFormat>
  *                                                       degeneracy_approx_csr.h:13-78 (push), degeneracy_approx_set.h:14-85 (pull)
  * boundary = one of boundary_function::{averageDegree, minDegree, probMinDegree, probMedianDegree}
